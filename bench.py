@@ -56,6 +56,8 @@ def parse():
     ap.add_argument("--math", default="tc3f16", choices=["tc3f16", "fp32", "tc1f16"])
     ap.add_argument("--ref-ddpm-sample", type=int, default=20, help="reference arm: DDPM steps timed per bench step")
     ap.add_argument("--no-extras", action="store_true", help="headline only (skip cfg2/cfg3/cfg4/eager/cpu legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the waveform the last timed step returned to DIR/wav.npy (float32; every rank's clips at N > 1)")
     return ap.parse_args()
 
 
@@ -108,6 +110,7 @@ def build_models(math_mode, ddpm_steps):
     import diffsvc_b200 as D
     from diffsvc_b200.hparams import hparams, DEFAULTS_44K
     hparams.clear(); hparams.update(DEFAULTS_44K); hparams["pndm_speedup"] = 1
+    torch.manual_seed(0)                     # the conditioning encoder's pitch embedding comes from the default generator
     sd = S.synth_diffnet_weights()
     dn = D.DiffNet(MEL, math_mode=math_mode)
     dn.load_state_dict(sd, strict=True)
@@ -376,6 +379,23 @@ def profile_traffic(B, T):
         return None, None
 
 
+DUMP_LIMIT_BYTES = 64_000_000 - 4096       # 64 MB for everything written, .npy headers included
+
+
+def dump_outputs(out_dir, wav):
+    """DIR/wav.npy: the [clips, samples] float32 waveform of the last timed step, so that two builds run with the same
+    arguments can be compared output for output.  The files stay within 64 MB in all: above that a fixed sample is
+    kept, every k-th sample of the flattened array, k the least stride that fits (the stride goes to DIR/wav_stride.npy)."""
+    import numpy as np
+    a = wav.detach().float().cpu().numpy()
+    stride = -(-a.nbytes // DUMP_LIMIT_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    if stride > 1:
+        a = a.reshape(-1)[::stride].copy()
+        np.save(os.path.join(out_dir, "wav_stride.npy"), np.array([stride], dtype=np.float64))
+    np.save(os.path.join(out_dir, "wav.npy"), a)
+
+
 def emit(line):
     """The ONE JSON line, on the real stdout (fd saved in main() before everything else was pointed at stderr)."""
     os.write(_REAL_STDOUT, (json.dumps(line) + "\n").encode())
@@ -427,7 +447,7 @@ def main():
     with torch.no_grad():
         ret0 = gd.fs2(hubert.cuda(), mel2ph.cuda(), None, None, f0.cuda().clone(), None, None, skip_decoder=True, infer=True)
     cond_d = ret0["decoder_inp"].transpose(1, 2).contiguous()
-    x0_d = torch.randn(B, 1, MEL, T, device="cuda")
+    x0_d = torch.randn(B, 1, MEL, T, generator=torch.Generator().manual_seed(2000 + rank)).cuda()   # same x_T every run
     f0hz_d = f0_hz.cuda()
 
     def step_device(i):
@@ -444,8 +464,8 @@ def main():
         return wav
 
     def timed(fn, n_warm, n_steps, sampler=None):
-        """ms per step (max over ranks of the per-rank sums) and every rank's own ms per step."""
-        tot = 0.0
+        """ms per step (max over ranks of the per-rank sums), every rank's own ms per step, what the last step returned."""
+        tot, out = 0.0, None
         for i in range(n_warm + n_steps):
             if dist is not None:
                 dist.barrier()
@@ -453,7 +473,7 @@ def main():
             if i == n_warm and sampler is not None:
                 sampler.start()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record(); fn(i); b.record()
+            a.record(); out = fn(i); b.record()
             torch.cuda.synchronize()
             if i >= n_warm:
                 tot += a.elapsed_time(b)
@@ -463,15 +483,17 @@ def main():
             every = [torch.empty_like(t) for _ in range(world)]
             dist.all_gather(every, t)
             per_rank = [float(v.item()) for v in every]
-        return max(per_rank), per_rank
+        return max(per_rank), per_rank, out
 
     with torch.no_grad():
         clk = ClockSampler(local)
         l0 = lib.dsvc_launch_count()
-        ms_dev, ranks_dev = timed(step_device, args.warmup, args.steps, clk)
+        ms_dev, ranks_dev, wav_dev = timed(step_device, args.warmup, args.steps, clk)
         clocks = clk.stop()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, (gathered if world > 1 else wav_dev).reshape(world * B, T * HOP))
         launches = (lib.dsvc_launch_count() - l0) // (args.warmup + args.steps) * args.steps
-        ms_e2e, ranks_e2e = timed(step_e2e, args.warmup, args.steps)
+        ms_e2e, ranks_e2e, _ = timed(step_e2e, args.warmup, args.steps)
         # sampler alone, and the two kernels of a layer alone (CUDA events on the launch stream, back to back)
         ms_sampler, _ = event_ms(lambda: gd.sample(x0_d, cond_d, NS, None, None, seed=3))
         h = gd.denoise_fn.handle()

@@ -1,8 +1,9 @@
 """Generate golden input/output vectors from the UNMODIFIED reference (CPU, fp32).
 
-Run once in the build container (where /root/reference exists):
+Run once, with DIFFSVC_REFERENCE_ROOT pointing at a checkout of the reference:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py                 # the small-size fixtures
+    python tests/golden/make_golden.py --only-full     # full_44k.npz (tests/test_oracle_vs_reference.py)
 
 It imports the reference's own `DiffNet`, `GaussianDiffusion` (incl. its FastSpeech2
 conditioning) and NSF-HiFiGAN `Generator`, builds them at SMALL sizes with seeded
@@ -297,7 +298,137 @@ def gen_pe():
     print("pe_small", ret["pitch_pred"].shape, float(ret["f0_denorm_pred"].max()))
 
 
+def full_pe_weights(shapes, seed=21):
+    """Seeded PitchExtractor weights for the key -> shape table of the full-size module: fan-in scaled convs and
+    projections, norm scales near 1, non-trivial BatchNorm statistics, and a predictor bias that puts log2(f0)
+    near 7 (~130 Hz).  Rebuilt from the table alone, so the comparison needs no copy of the reference's module."""
+    g = torch.Generator().manual_seed(seed)
+    sd = {}
+    for k, shape in shapes.items():
+        shape = tuple(int(s) for s in shape)
+        if k.endswith("num_batches_tracked"):
+            sd[k] = torch.zeros(shape, dtype=torch.long)
+        elif k.endswith("running_mean"):
+            sd[k] = 0.2 * torch.randn(shape, generator=g)
+        elif k.endswith("running_var"):
+            sd[k] = 0.5 + torch.rand(shape, generator=g)
+        elif k.endswith("pos_embed_alpha") or k.endswith("_float_tensor"):
+            sd[k] = torch.ones(shape)
+        elif k.endswith(".weight") and len(shape) >= 2:
+            sd[k] = torch.randn(shape, generator=g) / float(np.sqrt(np.prod(shape[1:])))
+        elif k.endswith(".weight"):
+            sd[k] = 1.0 + 0.1 * torch.randn(shape, generator=g)
+        else:
+            sd[k] = 0.1 * torch.randn(shape, generator=g)
+    sd["pitch_predictor.linear.bias"] = sd["pitch_predictor.linear.bias"] + torch.tensor([7.0, 0.0])
+    return sd
+
+
+def full_inputs():
+    """The inputs of tests/test_oracle_vs_reference.py, from their seeds."""
+    g = torch.Generator().manual_seed(1)
+    x = torch.randn(1, 1, 128, 96, generator=g)
+    cond = torch.randn(1, 256, 96, generator=g) * 0.5
+    noises = [torch.randn(1, 1, 128, 96, generator=g) for _ in range(3)]
+    g = torch.Generator().manual_seed(2)
+    T = 6
+    voc_mel = torch.randn(1, 128, T, generator=g) * 2 - 5
+    voc_f0 = O.synth_f0(1, T) + 100
+    voc_f0[0, 2] = 0
+    rand_ini = torch.rand(1, 9, generator=g)
+    sine_noise = torch.randn(1, T * 512, 9, generator=g)
+    g = torch.Generator().manual_seed(21)
+    pe_mel = torch.randn(2, 120, 80, generator=g) - 3.0
+    pe_mel[1, 100:] = 0
+    g = torch.Generator().manual_seed(4)
+    wav = (torch.rand(1, 30000, generator=g) * 2 - 1) * 0.3
+    return dict(x=x, cond=cond, noises=noises, voc_mel=voc_mel, voc_f0=voc_f0, rand_ini=rand_ini, sine_noise=sine_noise,
+                pe_mel=pe_mel, wav=wav)
+
+
+FULL_T = (999, 500, 0)
+
+
+def gen_full(hp):
+    """The reference's modules at the FULL 44.1 kHz config (config_nsf.yaml) on seeded weights and inputs that
+    tests/test_oracle_vs_reference.py rebuilds: reference outputs plus the key -> shape tables of its state dicts."""
+    inp = full_inputs()
+    d = {}
+    diffusion, net = rh.import_diffusion()
+    dn = net.DiffNet(128).eval()
+    dn.load_state_dict(O.synth_diffnet_weights(), strict=True)
+    gd = diffusion.GaussianDiffusion(None, 128, dn, timesteps=1000, K_step=1000, loss_type="l2",
+                                     spec_min=hp["spec_min"], spec_max=hp["spec_max"]).eval()
+    for k, v in dn.state_dict().items():
+        d["dn_shape/" + k] = np.asarray(v.shape, dtype=np.int64)
+    for k, v in gd.state_dict().items():                    # what a model checkpoint must load into (tests/test_dropin.py)
+        d["gd_shape/" + k] = np.asarray(v.shape, dtype=np.int64)
+    for i, tt in enumerate(FULL_T):
+        t = torch.tensor([tt])
+        noise = inp["noises"][i]
+        orig = diffusion.noise_like
+        diffusion.noise_like = lambda shape, device, repeat=False: noise
+        try:
+            with torch.no_grad():
+                d["dn_out/%d" % tt] = dn(inp["x"], t, inp["cond"]).numpy()
+                d["p_sample/%d" % tt] = gd.p_sample(inp["x"], t, inp["cond"]).numpy()
+        finally:
+            diffusion.noise_like = orig
+        for k in O.SCHEDULE_KEYS:
+            d["sched/" + k] = getattr(gd, k).numpy()
+
+    models = rh.import_nsf_models()
+    from modules.nsf_hifigan.env import AttrDict
+    gen = models.Generator(AttrDict(O.NSF_H_44K)).eval()
+    gen.remove_weight_norm()
+    gen.load_state_dict(O.synth_nsf_weights(O.NSF_H_44K))
+    for k, v in gen.state_dict().items():
+        d["nsf_shape/" + k] = np.asarray(v.shape, dtype=np.int64)
+    L = inp["voc_mel"].shape[-1] * 512
+    draws = iter([inp["rand_ini"], inp["sine_noise"], torch.zeros(1, L, 1)])   # models.py:192, :271, :322
+    o_rand, o_randn_like = torch.rand, torch.randn_like
+    torch.rand = lambda *a, **k: next(draws).clone()
+    torch.randn_like = lambda *a, **k: next(draws).clone()
+    try:
+        with torch.no_grad():
+            d["nsf/wav"] = gen(inp["voc_mel"], inp["voc_f0"]).numpy()
+    finally:
+        torch.rand, torch.randn_like = o_rand, o_randn_like
+
+    import modules.fastspeech.pe as pe_mod
+    m = pe_mod.PitchExtractor(n_mel_bins=80, conv_layers=2).eval()
+    shapes = {k: v.shape for k, v in m.state_dict().items()}
+    m.load_state_dict(full_pe_weights(shapes), strict=True)
+    for k, s in shapes.items():
+        d["pe_shape/" + k] = np.asarray(s, dtype=np.int64)
+    with torch.no_grad():
+        ret = m(inp["pe_mel"])
+    d["pe/pitch_pred"] = ret["pitch_pred"].numpy()
+    d["pe/f0_denorm_pred"] = ret["f0_denorm_pred"].numpy()
+
+    import modules.nsf_hifigan.nvSTFT as nv
+    nv.librosa_mel_fn = lambda sr, n_fft, n_mels, fmin, fmax: O.slaney_mel_basis(sr, n_fft, n_mels, fmin, fmax)
+    stft_now = torch.stft
+    nv.torch.stft = lambda *a, **k: stft_now(*a, **k) if "return_complex" in k else torch.view_as_real(stft_now(*a, return_complex=True, **k))
+    try:
+        stft = nv.STFT(hp["audio_sample_rate"], hp["audio_num_mel_bins"], hp["fft_size"], hp["win_size"], hp["hop_size"],
+                       hp["fmin"], hp["fmax"])
+        with torch.no_grad():
+            d["mel/out"] = stft.get_mel(inp["wav"]).numpy()
+    finally:
+        torch.stft = stft_now
+    for k in ("audio_sample_rate", "audio_num_mel_bins", "fft_size", "win_size", "hop_size", "fmin", "fmax"):
+        d["hp/" + k] = np.int64(hp[k])
+    d["hp/spec_min"] = np.asarray(hp["spec_min"], dtype=np.float32)
+    d["hp/spec_max"] = np.asarray(hp["spec_max"], dtype=np.float32)
+    np.savez_compressed(os.path.join(HERE, "full_44k.npz"), **d)
+    print("full_44k", {k: v.shape for k, v in d.items() if "shape/" not in k})
+
+
 def main():
+    if "--only-full" in sys.argv:
+        gen_full(rh.install())
+        return
     hp = rh.install(overrides=SMALL)
     if "--only-pe" in sys.argv:
         gen_pe()

@@ -6,7 +6,7 @@ the reference loads (SURVEY.md section 8c):
 
   native     the unmodified infer_tools.infer_tool under `diffsvc_b200.dropin.install()` on cuda:0 -- what a user
              of inference.ipynb / batch.py / flask_api.py gets after switching;
-  reference  the unmodified reference alone (baseline/_ref or /root/reference) on the CPU (`.cuda()` neutralised,
+  reference  the unmodified reference alone (DIFFSVC_REFERENCE_ROOT) on the CPU (`.cuda()` neutralised,
              CUDA hidden), the north_star's stated oracle.
 
 Host-side code that stays the reference's own (HuBERT, f0) is fed through its own hooks: HuBERT units come from
@@ -18,6 +18,12 @@ SineGen noise), so both arms compute the same function of the same numbers.
 
     python tests/svc_e2e.py make  <workdir> [--seconds 3] [--k-step 1000]
     python tests/svc_e2e.py run   <workdir> --arm native|reference --acc 20 [--use-pe] [--patch-after-infer] --out x.npz
+    python tests/svc_e2e.py golden <workdir> --seconds 3 --k-step 1000 --acc 20 --out tests/golden/svc_infer_plms.npz
+
+`golden` runs the reference arm alone with the draws the native arm takes from its seeded generator, and stores
+what `Svc.infer` fed the model (the batch of `Svc.pre`) next to everything tests/test_svc_infer_gpu.py compares.
+The checkpoints hold the seeded weights of synthetic.py (plus a seeded pitch embedding), so the native side can be
+rebuilt from the repository alone.
 """
 import argparse
 import json
@@ -30,6 +36,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(HERE, "golden"))
+
+SEED = 1234
+NATIVE_DRAW_SEED = 99
 
 NSF_H = {"resblock": "1", "upsample_rates": [8, 8, 2, 2, 2], "upsample_kernel_sizes": [16, 16, 4, 4, 4],
          "upsample_initial_channel": 512, "resblock_kernel_sizes": [3, 7, 11],
@@ -60,7 +69,7 @@ def fake_f0(n_frames, hparams):
     return f0, f0_to_coarse(f0, hparams)
 
 
-def make(workdir, seconds, k_step, seed=1234):
+def make(workdir, seconds, k_step, seed=SEED):
     """Synthetic project: config.yaml, model / pe / vocoder checkpoint files, a wav and its HuBERT-units cache."""
     import torch
     import yaml
@@ -87,8 +96,10 @@ def make(workdir, seconds, k_step, seed=1234):
     diffusion, net = rh.import_diffusion()
     gd = diffusion.GaussianDiffusion(None, 128, net.DiffNet(128), timesteps=hp["timesteps"], K_step=int(k_step),
                                      loss_type=hp["diff_loss_type"], spec_min=hp["spec_min"], spec_max=hp["spec_max"])
-    with torch.no_grad():                                 # zero-initialised in the reference (net.py:110)
-        gd.denoise_fn.output_projection.weight.normal_(0.0, 0.05)
+    import synthetic as S
+    with torch.no_grad():                                 # seeded weights the native side rebuilds (synthetic.py)
+        gd.denoise_fn.load_state_dict(S.synth_diffnet_weights(), strict=True)
+        gd.fs2.pitch_embed.weight.copy_(pitch_embed_weight(hp["hidden_size"]))
     torch.save({"state_dict": {"model." + k: v for k, v in gd.state_dict().items()}},
                os.path.join(ck, "proj", "model_ckpt_steps_1.ckpt"))
     import modules.fastspeech.pe as ref_pe
@@ -97,7 +108,8 @@ def make(workdir, seconds, k_step, seed=1234):
                os.path.join(ck, "pe", "model_ckpt_steps_1.ckpt"))
     models = rh.import_nsf_models()
     gen = models.Generator(models.AttrDict(NSF_H))        # weight-norm form: weight_g / weight_v keys
-    torch.save({"generator": gen.state_dict()}, os.path.join(ck, "nsf_hifigan", "model"))
+    torch.save({"generator": weight_norm_form(gen.state_dict(), S.synth_nsf_weights(S.NSF_H_44K))},
+               os.path.join(ck, "nsf_hifigan", "model"))
     with open(os.path.join(ck, "nsf_hifigan", "config.json"), "w") as f:
         json.dump(NSF_H, f)
     torch.save({}, os.path.join(ck, "hubert", "hubert_soft.pt"))    # globbed by Hubertencoder; the loader is stubbed
@@ -108,6 +120,27 @@ def make(workdir, seconds, k_step, seed=1234):
     n_units = max(2, int(len(wav) / 44100 * 50))          # HuBERT-soft: 50 units / s, 256 wide
     g = torch.Generator().manual_seed(seed + 1)
     np.save(os.path.join(workdir, "raw", "clip.npy"), (torch.randn(n_units, 256, generator=g) * 0.5).numpy())
+
+
+def pitch_embed_weight(hidden=256):
+    """The seeded FastSpeech2 pitch embedding of the synthetic checkpoint (padding row 0 zero)."""
+    import torch
+    w = torch.randn(300, hidden, generator=torch.Generator().manual_seed(SEED + 2)) * hidden ** -0.5
+    w[0] = 0
+    return w
+
+
+def weight_norm_form(gen_sd, folded):
+    """A weight-norm generator state dict (weight_g / weight_v, dim 0) whose folded weights are `folded`."""
+    out = {}
+    for k, v in gen_sd.items():
+        if k.endswith("weight_v"):
+            w = folded[k[:-2]]
+            out[k] = w.clone()
+            out[k[:-1] + "g"] = w.reshape(w.shape[0], -1).norm(dim=1).reshape(v.shape[:1] + (1,) * (v.dim() - 1))
+        elif not k.endswith("weight_g"):
+            out[k] = folded[k].clone()
+    return out
 
 
 def _soundfile_double():
@@ -157,7 +190,37 @@ class _Draws:
         return fallback()
 
 
-def run(workdir, arm, acc, use_pe, patch_after_infer, out, draws_in):
+class _SeededDraws:
+    """The native arm's draws regenerated in its order from its seeded generator: x_T, then (DDPM) every step's noise
+    as one tensor, then the vocoder's initial phases and sine noise.  Other draws (the NSF source's unused noise
+    branch) fall through."""
+
+    def __init__(self, torch, k_step, ddpm):
+        self.g = torch.Generator().manual_seed(NATIVE_DRAW_SEED)
+        self.randn, self.rand = torch.randn, torch.rand          # the unpatched functions
+        self.k_step, self.ddpm, self.x_shape, self.queue, self.pos = k_step, ddpm, None, [], 0
+        self.expected = 1 + (k_step if ddpm else 0) + 2
+
+    def replay(self, torch, kind, shape, device, fallback):
+        shape = tuple(shape)
+        if kind == "randn" and self.x_shape is None and len(shape) == 4 and shape[:3] == (1, 1, 128):
+            self.x_shape = shape
+            draw = self.randn(shape, generator=self.g)
+            if self.ddpm:
+                self.queue = list(self.randn((self.k_step,) + shape, generator=self.g))
+        elif kind == "randn" and shape == self.x_shape and self.queue:
+            draw = self.queue.pop(0)
+        elif kind == "rand" and shape == (1, 9):
+            draw = self.rand(shape, generator=self.g)
+        elif kind == "randn" and len(shape) == 3 and shape[0] == 1 and shape[2] == 9:
+            draw = self.randn(shape, generator=self.g)
+        else:
+            return fallback()
+        self.pos += 1
+        return draw.to(device)
+
+
+def run(workdir, arm, acc, use_pe, patch_after_infer, out, draws_in, golden=False):
     os.chdir(workdir)
     if arm == "reference":
         os.environ["CUDA_VISIBLE_DEVICES"] = ""
@@ -195,7 +258,7 @@ def run(workdir, arm, acc, use_pe, patch_after_infer, out, draws_in):
     svc.model.out2mel = out2mel
     k_step = int(hparams["K_step"])
     if arm == "native":
-        g = torch.Generator().manual_seed(99)
+        g = torch.Generator().manual_seed(NATIVE_DRAW_SEED)
         draws = []
         orig_forward = type(svc.model).forward
 
@@ -233,7 +296,7 @@ def run(workdir, arm, acc, use_pe, patch_after_infer, out, draws_in):
         if draws_in:
             rec = np.load(draws_in, allow_pickle=True)
             recorded = [(str(k), rec["d%d" % i]) for i, k in enumerate(rec["kinds"])]
-        dr = _Draws(recorded)
+        dr = _SeededDraws(torch, k_step, not (acc and acc > 1)) if golden else _Draws(recorded)
         o_randn, o_rand, o_randn_like = torch.randn, torch.rand, torch.randn_like
 
         def randn(*size, **kw):
@@ -253,6 +316,23 @@ def run(workdir, arm, acc, use_pe, patch_after_infer, out, draws_in):
             captured["mel_pred"] = np.asarray(mel); captured["f0_voc"] = np.asarray(kw["f0"])
             return orig(mel, **kw)
         svc.vocoder.spec2wav = call
+        if golden:                                 # what Svc.infer fed the model, and the prediction after_infer received
+            orig_forward = type(svc.model).forward
+
+            def forward(self, hubert, mel2ph=None, spk_embed=None, f0=None, uv=None, energy=None, ref_mels=None, **kw):
+                for k, v in (("hubert", hubert), ("mel2ph", mel2ph), ("f0", f0), ("uv", uv), ("energy", energy),
+                             ("ref_mels", ref_mels)):
+                    captured["in_" + k] = v.detach().clone().numpy()
+                return orig_forward(self, hubert, mel2ph=mel2ph, spk_embed=spk_embed, f0=f0, uv=uv, energy=energy,
+                                    ref_mels=ref_mels, **kw)
+            type(svc.model).forward = forward
+            orig_after = svc.after_infer
+
+            def after_infer(prediction, singer, in_path):
+                captured["in_mels"] = np.asarray(prediction["mels"]).copy()
+                captured["in_f0_gt"] = np.asarray(prediction["f0_gt"]).copy()
+                return orig_after(prediction, singer, in_path)
+            svc.after_infer = after_infer
     with torch.no_grad():
         f0_gt, f0_pred, wav = svc.infer("raw/clip.wav", 0, acc, use_pe=use_pe, use_crepe=False, **kwargs)
     res = {"f0_gt": np.asarray(f0_gt), "f0_pred": np.asarray(f0_pred), "wav": np.asarray(wav), **captured}
@@ -263,14 +343,19 @@ def run(workdir, arm, acc, use_pe, patch_after_infer, out, draws_in):
         from diffsvc_b200 import _lib
         res["launches"] = np.array(_lib.load().dsvc_launch_count())
     else:
-        res["replayed"] = np.array(dr.pos); res["recorded"] = np.array(len(recorded))
-    np.savez(out, **res)
+        res["replayed"] = np.array(dr.pos); res["recorded"] = np.array(dr.expected if golden else len(recorded))
+    if golden:
+        res.update(acc=np.int64(acc), k_step=np.int64(k_step), spec_min=np.asarray(hparams["spec_min"], np.float32),
+                   spec_max=np.asarray(hparams["spec_max"], np.float32))
+        np.savez_compressed(out, **res)
+    else:
+        np.savez(out, **res)
     print("SVC_E2E_OK", arm, {k: getattr(v, "shape", None) for k, v in res.items() if not k.startswith("d")})
 
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("cmd", choices=["make", "run"])
+    ap.add_argument("cmd", choices=["make", "run", "golden"])
     ap.add_argument("workdir")
     ap.add_argument("--seconds", type=float, default=3.0)
     ap.add_argument("--k-step", type=int, default=1000)
@@ -283,6 +368,9 @@ if __name__ == "__main__":
     a = ap.parse_args()
     if a.cmd == "make":
         make(os.path.abspath(a.workdir), a.seconds, a.k_step)
+    elif a.cmd == "golden":
+        make(os.path.abspath(a.workdir), a.seconds, a.k_step)
+        run(os.path.abspath(a.workdir), "reference", a.acc, False, False, os.path.abspath(a.out), None, golden=True)
     else:
         run(os.path.abspath(a.workdir), a.arm, a.acc, a.use_pe, a.patch_after_infer, os.path.abspath(a.out),
             os.path.abspath(a.draws) if a.draws else None)
