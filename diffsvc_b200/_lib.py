@@ -148,6 +148,7 @@ SYMBOLS = [
     ("dsvc_sample_ddpm", C.c_int, [_VP, _VP, C.c_int32, _VP, C.c_uint64, _VP]),
     ("dsvc_sample_plms", C.c_int, [_VP, _VP, C.c_int32, C.c_int32, _VP]),
     ("dsvc_nsf_create", C.c_int, [C.POINTER(_VP), C.POINTER(NsfConfig), C.POINTER(NsfWeights), _VP]),
+    ("dsvc_nsf_create_ex", C.c_int, [C.POINTER(_VP), C.POINTER(NsfConfig), C.c_int32, C.POINTER(NsfWeights), _VP]),
     ("dsvc_nsf_destroy", None, [_VP]),
     ("dsvc_nsf_forward", C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_uint64, C.c_float, _VP, C.c_int32, C.c_int32, _VP]),
     ("dsvc_mel_frames", C.c_int64, [C.POINTER(MelConfig), C.c_int64]),

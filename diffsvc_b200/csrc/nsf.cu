@@ -1,6 +1,6 @@
 // NSF-HiFiGAN generator: harmonic-plus-noise source, transposed-conv upsampling, MRF residual blocks.
 // Reference: modules/nsf_hifigan/models.py:148-387 (SineGen :148, SourceModuleHnNSF :277,
-// ResBlock1 :33, effective Generator :325), called from network/vocoders/nsf_hifigan.py:36-72.
+// ResBlock1 :33, ResBlock2 :73, effective Generator :325), called from network/vocoders/nsf_hifigan.py:36-72.
 //
 // Activations are channels-last fp32 [B][L][C]; every Conv1d / ConvTranspose1d is an implicit GEMM
 // (simt_gemm.cuh) with the LeakyReLU fused into the operand load and bias / residual / MRF
@@ -254,6 +254,7 @@ struct ConvW {
   // tcgen05 path (ResBlock convs whose channel count tiles by 64): fp16 hi/lo weights [K][Cout][Cin] + their TMA maps
   bool tc = false;
   int kb = 0;                 // narrow convs (Cin = Cout = 32 / 16) on tcgen05 (tc_narrow.cuh): operand rows of Cin fp16
+  int pad = NW_PAD;           // ... and the rows their activation window reaches either side of a tile
   F16Pair h16;
   CUtensorMap bh, bl, b32h, b32l, b64h, b64l;   // weight boxes of 128 / 32 / 64 rows (tc_gemm.cuh, tc_pair.cuh)
 };
@@ -279,9 +280,10 @@ struct NsfStageMaps {          // activation-plane TMA maps of one upsample stag
 
 struct dsvc_nsf {
   dsvc_nsf_config cfg;
+  int resblock = 1;            // 1: ResBlock1 (convs1 / convs2 pairs), 2: ResBlock2 (two convs, c1 only)
   int hop = 1;
   bool tc_enabled = true;      // DSVC_NSF_MATH=fp32 forces the FFMA path everywhere
-  bool narrow_ok = true;       // the 32- / 16-channel stages can take tc_narrow.cuh (window reach, DSVC_NSF_NARROW)
+  int narrow_pad = NW_PAD;     // window half-height of tc_narrow.cuh for the 32- / 16-channel stages; 0 = FFMA GEMM
   PlaneBuf PX, PA, PT;         // leaky_relu'ed operand planes: stage input, ResBlock state, conv1 output
   std::vector<NsfStageMaps> smaps;
   int maps_B = 0, maps_T = 0;
@@ -382,8 +384,10 @@ static int conv_same_tc(const ConvW& c, const TcGemmMaps& in, EpiVoc::Params e, 
   TcGemmMaps g = in;
   g.b_hi = c.bh; g.b_lo = c.bl; g.b32_hi = c.b32h; g.b32_lo = c.b32l; g.b64_hi = c.b64h; g.b64_lo = c.b64l;
   e.bias = c.b.as<float>(); e.Lout = L; e.Cout = c.Cout; e.wscale = c.h16.inv_scale;
-  if (c.kb == 32) return tc_narrow_launch<32>(in.a_hi, in.a_lo, c.b32h, c.b32l, e, B, L, c.K, dil, s);
-  if (c.kb == 16) return tc_narrow_launch<16>(in.a_hi, in.a_lo, c.b32h, c.b32l, e, B, L, c.K, dil, s);
+  if (c.kb == 32 && c.pad == NW_PAD) return tc_narrow_launch<32, NW_PAD>(in.a_hi, in.a_lo, c.b32h, c.b32l, e, B, L, c.K, dil, s);
+  if (c.kb == 16 && c.pad == NW_PAD) return tc_narrow_launch<16, NW_PAD>(in.a_hi, in.a_lo, c.b32h, c.b32l, e, B, L, c.K, dil, s);
+  if (c.kb == 32) return tc_narrow_launch<32, NW_PAD_WIDE>(in.a_hi, in.a_lo, c.b32h, c.b32l, e, B, L, c.K, dil, s);
+  if (c.kb == 16) return tc_narrow_launch<16, NW_PAD_WIDE>(in.a_hi, in.a_lo, c.b32h, c.b32l, e, B, L, c.K, dil, s);
   return tc_launch<EpiVoc>(g, e, B, L, c.Cin, c.Cout, c.K, dil, 3, s);
 }
 
@@ -391,16 +395,21 @@ static int conv_same_tc(const ConvW& c, const TcGemmMaps& in, EpiVoc::Params e, 
 // on the FFMA GEMM (their weights are kept in both forms).
 static bool nsf_tc_channels(const dsvc_nsf* h, int ch) {
   if (ch % 64 == 0) return true;
-  return (ch == 32 || ch == 16) && h->narrow_ok;
+  return (ch == 32 || ch == 16) && h->narrow_pad > 0;
 }
-// ... when every ResBlock conv's taps stay inside the kernel's activation window (k/2 * dilation <= NW_PAD rows)
-static bool nsf_narrow_fits(const dsvc_nsf_config& cfg) {
+// ... when every ResBlock conv's taps stay inside the kernel's activation window (k/2 * dilation <= pad rows): the
+// 192-row window (pad 32) when it fits; for ResBlock2 generators the 256-row one (pad 64) next.  ResBlock1 generators
+// that reach past 32 rows stay on FFMA.  Returns the pad, 0 for the FFMA GEMM.
+static int nsf_narrow_pad(const dsvc_nsf_config& cfg, int resblock) {
   const char* e = getenv("DSVC_NSF_NARROW");
-  if (e && atoi(e) == 0) return false;
+  if (e && atoi(e) == 0) return 0;
+  int reach = 0;
   for (int j = 0; j < cfg.num_kernels; ++j)
     for (int m = 0; m < cfg.num_dilations; ++m)
-      if ((cfg.resblock_kernel_sizes[j] / 2) * std::max(1, cfg.resblock_dilation_sizes[j][m]) > NW_PAD) return false;
-  return true;
+      reach = std::max(reach, (cfg.resblock_kernel_sizes[j] / 2) * std::max(1, cfg.resblock_dilation_sizes[j][m]));
+  if (reach <= NW_PAD) return NW_PAD;
+  if (resblock == 2 && reach <= NW_PAD_WIDE) return NW_PAD_WIDE;
+  return 0;
 }
 
 // (re)build the activation-plane maps for a (B, T) shape
@@ -415,8 +424,8 @@ static int nsf_build_maps(dsvc_nsf* h, int B, int T) {
     NsfStageMaps& m = h->smaps[i];
     m.tc = h->tc_enabled && nsf_tc_channels(h, ch);
     if (!m.tc) continue;
-    // narrow stages: operand rows of `ch` fp16 and one 192-row window per tile (tc_narrow.cuh); else [128 x 64] tiles
-    const int kb = ch < 64 ? ch : TC_BK, box_rows = ch < 64 ? NW_WIN : TC_BM;
+    // narrow stages: operand rows of `ch` fp16 and one 192- / 256-row window per tile (tc_narrow.cuh); else [128 x 64] tiles
+    const int kb = ch < 64 ? ch : TC_BK, box_rows = ch < 64 ? nw_rows(h->narrow_pad) : TC_BM;
     auto planes = [&](TcGemmMaps& g, const PlaneBuf& pb) -> int {
       DSVC_TRY(tc_make_a_map(&g.a_hi, pb.hi.as<__half>(), B, len, ch, box_rows, kb));
       DSVC_TRY(tc_make_a_map(&g.a_lo, pb.lo.as<__half>(), B, len, ch, box_rows, kb));
@@ -430,13 +439,56 @@ static int nsf_build_maps(dsvc_nsf* h, int B, int T) {
   return DSVC_OK;
 }
 
+// MRF of ResBlock2 generators (models.py:86-91): per kernel j, x1 = c0(lrelu(xu)) + xu, xs (+)= c1(lrelu(x1)) + x1,
+// the last j divides by num_kernels.  On tcgen05, conv 0 reads PX (lrelu(xu), written once per stage) and its epilogue
+// writes x1 and the planes of lrelu(x1) to PA, which conv 1 reads.  On the FFMA GEMM the LeakyReLU is on the operand load.
+static int nsf_mrf_resblock2(dsvc_nsf* h, int i, const float* xu, float* xs, int B, int lout, cudaStream_t s) {
+  const dsvc_nsf_config& cfg = h->cfg;
+  const int nk = cfg.num_kernels, C = h->c1[i * nk * 2]->Cout;
+  float* x1 = h->bufR0.as<float>();
+  const NsfStageMaps& sm = h->smaps[i];
+  if (sm.tc) {
+    const size_t n4 = (size_t)B * lout * C / 4;
+    act_split_kernel<<<(unsigned)((n4 + 255) / 256), 256, 0, s>>>(xu, h->PX.hi.as<__half>(), h->PX.lo.as<__half>(), n4, 0.1f);
+    DSVC_LAUNCH_CHECK();
+  }
+  for (int j = 0; j < nk; ++j) {
+    const ConvW& c0 = *h->c1[(i * nk + j) * 2];
+    const ConvW& c1 = *h->c1[(i * nk + j) * 2 + 1];
+    const int d0 = cfg.resblock_dilation_sizes[j][0], d1 = cfg.resblock_dilation_sizes[j][1];
+    const int acc = j > 0 ? 1 : 0;
+    const float div = (j + 1 == nk) ? (float)nk : 1.0f;
+    if (sm.tc) {
+      EpiVoc::Params e0{};
+      e0.res = xu; e0.out = x1; e0.act = h->PA.view(true); e0.div = 1.0f; e0.slope = 0.1f;
+      DSVC_TRY(conv_same_tc(c0, sm.px, e0, B, lout, d0, s));
+      EpiVoc::Params e1{};
+      e1.res = x1; e1.out = xs; e1.accumulate = acc; e1.div = div; e1.slope = 0.1f;
+      DSVC_TRY(conv_same_tc(c1, sm.pa, e1, B, lout, d1, s));
+    } else {
+      DSVC_TRY(conv_same(c0, xu, x1, xu, B, lout, d0, 0.1f, 0, 1.0f, s));
+      DSVC_TRY(conv_same(c1, x1, xs, x1, B, lout, d1, 0.1f, acc, div, s));
+    }
+  }
+  return DSVC_OK;
+}
+
 }  // namespace dsvc
 
 extern "C" {
 
 int dsvc_nsf_create(dsvc_nsf_t** out, const dsvc_nsf_config* cfg, const dsvc_nsf_weights* w, void* stream) {
+  return dsvc_nsf_create_ex(out, cfg, 1, w, stream);
+}
+
+int dsvc_nsf_create_ex(dsvc_nsf_t** out, const dsvc_nsf_config* cfg, int32_t resblock, const dsvc_nsf_weights* w,
+                       void* stream) {
   DSVC_REQUIRE(out && cfg && w, "dsvc_nsf_create: null argument");
   DSVC_TRY(require_device());
+  DSVC_REQUIRE(resblock == 1 || resblock == 2, "resblock %d: expected 1 (ResBlock1) or 2 (ResBlock2)", resblock);
+  DSVC_REQUIRE(resblock == 1 || (cfg->num_dilations == 2 && !w->convs2_w && !w->convs2_b),
+               "ResBlock2 takes exactly two convs per block (num_dilations 2, got %d) in convs1_*, and convs2_* NULL",
+               cfg->num_dilations);
   DSVC_REQUIRE(cfg->num_upsamples >= 1 && cfg->num_upsamples <= DSVC_NSF_MAX_STAGES, "num_upsamples %d out of range", cfg->num_upsamples);
   DSVC_REQUIRE(cfg->num_kernels >= 1 && cfg->num_kernels <= DSVC_NSF_MAX_KERNELS, "num_kernels %d out of range", cfg->num_kernels);
   DSVC_REQUIRE(cfg->num_dilations >= 1 && cfg->num_dilations <= DSVC_NSF_MAX_DILATIONS, "num_dilations %d out of range", cfg->num_dilations);
@@ -444,10 +496,11 @@ int dsvc_nsf_create(dsvc_nsf_t** out, const dsvc_nsf_config* cfg, const dsvc_nsf
   cudaStream_t s = (cudaStream_t)stream;
   std::unique_ptr<dsvc_nsf> h(new dsvc_nsf());
   h->cfg = *cfg;
+  h->resblock = resblock;
   {
     const char* ev = getenv("DSVC_NSF_MATH");
     h->tc_enabled = !(ev && strcmp(ev, "fp32") == 0);
-    h->narrow_ok = nsf_narrow_fits(*cfg);
+    h->narrow_pad = nsf_narrow_pad(*cfg, resblock);
   }
   const int ns = cfg->num_upsamples, nk = cfg->num_kernels, nd = cfg->num_dilations, dim = cfg->harmonic_num + 1;
   int ch = cfg->upsample_initial_channel;
@@ -493,10 +546,13 @@ int dsvc_nsf_create(dsvc_nsf_t** out, const dsvc_nsf_config* cfg, const dsvc_nsf
         const int k = cfg->resblock_kernel_sizes[j];
         DSVC_REQUIRE(k % 2 == 1, "resblock kernel size %d must be odd", k);
         h->c1.emplace_back(new ConvW());
-        h->c2.emplace_back(new ConvW());
         const bool tc = h->tc_enabled && nsf_tc_channels(h.get(), cout);
         DSVC_TRY(upload_conv(*h->c1[idx], w->convs1_w[idx], w->convs1_b[idx], cout, cout, k, s, tc));
+        h->c1[idx]->pad = h->narrow_pad;
+        if (resblock == 2) continue;                   // ResBlock2: resblocks.{i*nk+j}.convs.{m} only
+        h->c2.emplace_back(new ConvW());
         DSVC_TRY(upload_conv(*h->c2[idx], w->convs2_w[idx], w->convs2_b[idx], cout, cout, k, s, tc));
+        h->c2[idx]->pad = h->narrow_pad;
       }
     ch = cout;
   }
@@ -614,7 +670,9 @@ int dsvc_nsf_forward(dsvc_nsf_t* h, const float* mel, const float* f0, const flo
       DSVC_LAUNCH_CHECK();
     }
     // MRF: xs = sum_j ResBlock1_j(xu) / num_kernels
-    if (h->smaps[i].tc) {
+    if (h->resblock == 2) {
+      DSVC_TRY(nsf_mrf_resblock2(h, i, xu, xs, B, lout, s));
+    } else if (h->smaps[i].tc) {
       // tcgen05 path: every conv reads fp16 (hi, lo) planes of leaky_relu(.) written by the producing epilogue
       const NsfStageMaps& sm = h->smaps[i];
       const size_t n4 = (size_t)B * lout * up.Cout / 4;

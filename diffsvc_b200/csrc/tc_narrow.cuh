@@ -8,12 +8,14 @@
 // 256-frame tile is a CTA launch; above ~275 mel frames that lost to the FFMA GEMM.  Here
 //   * the conv's whole weight set ([wh ; wl] per tap: taps x 4 KB at C = 32) is loaded into shared memory ONCE per CTA,
 //   * a tile's activations are loaded ONCE: a window of 192 rows (the 128 output frames +- 32: every tap of every
-//     ResBlock conv, k <= 11 x dilation <= 5, reaches at most 25 rows out), hi and lo planes, 24 KB -- and each tap's
+//     ResBlock1 conv, k <= 11 x dilation <= 5, reaches at most 25 rows out) or 256 rows (+- 64, for ResBlock2
+//     dilations up to 12), hi and lo planes, 24 / 32 KB at C = 32 -- and each tap's
 //     operand is that window at a row offset: the UMMA descriptor's start address moves by (tap - taps/2) * dil rows
 //     (the swizzle XOR is a function of the absolute shared-memory address, so any row offset reads consistently);
 //     rows outside [0, L) are zero-filled by the TMA unit = the conv's zero padding,
-//   * a CTA loops over frame tiles (two windows in flight), and two CTAs share an SM (111 KB / 64 TMEM columns each),
-//     so one CTA's epilogue overlaps the other's MMAs without any role specialisation.
+//   * a CTA loops over frame tiles (two windows in flight), and two CTAs share an SM (<= 111 KB / 64 TMEM columns
+//     each: every 192-row case, and the 256-row window up to k = 7 at C = 32), so one CTA's epilogue overlaps the
+//     other's MMAs without any role specialisation.
 // Operand rows are C fp16 = 64 / 32 bytes: SWIZZLE_64B / 32B tiles (umma_desc_k<C>), K per tap = C = 2 / 1 MMA K-steps.
 // The 3-pass product keeps its two-MMA form: xh * [wh ; wl] (N = 2C) and xl * wh (N = C) into accumulator columns
 // [0, C) | [C, 2C).  Epilogue: the shared tc_epilogue / EpiVoc functor on a C-wide tile.
@@ -22,26 +24,32 @@
 
 namespace dsvc {
 
-constexpr int NW_WIN = 192;   // window rows per tile
-constexpr int NW_PAD = 32;    // of them before the tile's first frame (>= (taps / 2) * dil of every narrow conv)
+// The window is TC_BM output frames plus PAD rows either side; PAD >= (taps / 2) * dil of every conv it runs.
+// Two instances: PAD 32 (192 rows; every ResBlock1 conv of the shipped configs) and PAD 64 (256 rows, the TMA box
+// height limit; ResBlock2 dilations up to 12 at kernel 7 reach 36 rows).
+constexpr int NW_PAD = 32;        // the 192-row window
+constexpr int NW_PAD_WIDE = 64;   // the 256-row window
+constexpr int nw_rows(int pad) { return TC_BM + 2 * pad; }
 
-template <int C> struct NarrowCfg {
+template <int C, int PAD> struct NarrowCfg {
+  static constexpr int ROWS = nw_rows(PAD);                // window rows per tile
   static constexpr int ROWB = C * 2;                       // bytes per operand row
   static constexpr int W_TAP = 2 * C * ROWB;               // [wh ; wl] of one tap
-  static constexpr int WIN = NW_WIN * ROWB;                // one plane of one window
+  static constexpr int WIN = ROWS * ROWB;                  // one plane of one window
   static constexpr int SLAB = 4 * 32 * (C + 4) * 4;        // epilogue staging
   static constexpr int BARS = 128;
   static int smem(int taps) { return taps * W_TAP + 4 * WIN + BARS + SLAB + 1024; }
 };
 
-template <int C>
+template <int C, int PAD>
 __global__ void __launch_bounds__(TC_THREADS, 2)
 tc_narrow_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
                  const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl,
                  const EpiVoc::Params ep, int L, int taps, int dil, int tiles_per_item, int n_tiles) {
 #if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ >= 1000)
-  using Cfg = NarrowCfg<C>;
+  using Cfg = NarrowCfg<C, PAD>;
   static_assert(C == 32 || C == 16, "narrow convs: 32 or 16 channels");
+  static_assert(Cfg::ROWS <= 256, "a window is one TMA box: at most 256 rows");
   pdl_launch_dependents();
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -79,11 +87,11 @@ tc_narrow_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant
   uint32_t tmem_base;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
 
-  auto load_window = [&](int t, int buf) {           // one elected lane: the 192-row window of frame tile t, both planes
+  auto load_window = [&](int t, int buf) {           // one elected lane: the window of frame tile t, both planes
     const int b = t / tiles_per_item, m0 = (t - b * tiles_per_item) * TC_BM;
     mbar_expect_tx(a_full(buf), 2u * Cfg::WIN);
-    tma_load_3d(&tmAh, a_full(buf), win(buf, 0), 0, m0 - NW_PAD, b);
-    tma_load_3d(&tmAl, a_full(buf), win(buf, 1), 0, m0 - NW_PAD, b);
+    tma_load_3d(&tmAh, a_full(buf), win(buf, 0), 0, m0 - PAD, b);
+    tma_load_3d(&tmAl, a_full(buf), win(buf, 1), 0, m0 - PAD, b);
   };
 
   if (warp == 0) {
@@ -119,7 +127,7 @@ tc_narrow_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant
       tc_fence_after();
       if (elect_one_sync()) {
         for (int tap = 0; tap < taps; ++tap) {
-          const uint32_t row = (uint32_t)(NW_PAD + (tap - (taps >> 1)) * dil) * Cfg::ROWB;
+          const uint32_t row = (uint32_t)(PAD + (tap - (taps >> 1)) * dil) * Cfg::ROWB;
           const uint64_t ah = umma_desc_k<C>(win(buf, 0) + row), al = umma_desc_k<C>(win(buf, 1) + row);
           const uint64_t wd = umma_desc_k<C>(w_tap(tap));
 #pragma unroll
@@ -155,21 +163,31 @@ tc_narrow_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant
 #endif
 }
 
-template <int C>
+template <int C, int PAD>
 int tc_narrow_launch(const CUtensorMap& ah, const CUtensorMap& al, const CUtensorMap& bh, const CUtensorMap& bl,
                      const EpiVoc::Params& e, int B, int L, int taps, int dil, cudaStream_t s) {
-  DSVC_REQUIRE(taps >= 1 && (taps / 2) * dil <= NW_PAD && (taps / 2) * dil + TC_BM <= NW_WIN - NW_PAD,
-               "narrow conv: %d taps x dilation %d reach beyond the %d-row window", taps, dil, NW_WIN);
-  const int smem = NarrowCfg<C>::smem(taps);
-  DSVC_TRY((ensure_dyn_smem<tc_narrow_kernel<C>>(smem)));
+  DSVC_REQUIRE(taps >= 1 && taps < 64 && (taps / 2) * dil <= PAD,
+               "narrow conv: %d taps x dilation %d reach beyond the %d-row window", taps, dil, nw_rows(PAD));
+  const int smem = NarrowCfg<C, PAD>::smem(taps);
+  DSVC_TRY((ensure_dyn_smem<tc_narrow_kernel<C, PAD>>(smem)));
   static const int sms = [] {
     int dev = 0, n = 148;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
     return n > 0 ? n : 148;
   }();
+  // resident CTAs per SM at this tap count: 2 up to ~113 KB of shared memory (every 192-row case, the 256-row
+  // window up to k = 7 at C = 32), else 1 -- a persistent grid larger than what is resident only queues
+  static std::atomic<int> occ_by_taps[64];
+  int occ = occ_by_taps[taps].load(std::memory_order_relaxed);
+  if (occ == 0) {
+    DSVC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, tc_narrow_kernel<C, PAD>, TC_THREADS, smem));
+    DSVC_REQUIRE(occ >= 1, "narrow conv: %d bytes of shared memory do not fit an SM", smem);
+    occ = occ < 2 ? occ : 2;
+    occ_by_taps[taps].store(occ, std::memory_order_relaxed);
+  }
   const int per_item = ceil_div(L, TC_BM), n_tiles = per_item * B;
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(n_tiles < 2 * sms ? n_tiles : 2 * sms, 1, 1);
+  cfg.gridDim = dim3(n_tiles < occ * sms ? n_tiles : occ * sms, 1, 1);
   cfg.blockDim = dim3(TC_THREADS);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = s;
@@ -178,7 +196,7 @@ int tc_narrow_launch(const CUtensorMap& ah, const CUtensorMap& al, const CUtenso
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  DSVC_CUDA(cudaLaunchKernelEx(&cfg, tc_narrow_kernel<C>, ah, al, bh, bl, e, L, taps, dil, per_item, n_tiles));
+  DSVC_CUDA(cudaLaunchKernelEx(&cfg, tc_narrow_kernel<C, PAD>, ah, al, bh, bl, e, L, taps, dil, per_item, n_tiles));
   DSVC_LAUNCH_CHECK();
   return DSVC_OK;
 }

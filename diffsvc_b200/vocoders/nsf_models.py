@@ -31,6 +31,47 @@ def fold_weight_norm(sd):
     return out
 
 
+def resblock_type(h):
+    """models.py:337 / modules/hifigan/hifigan.py:119: ResBlock1 for '1', ResBlock2 for anything else.  A missing
+    key or an integer 1 also mean ResBlock1."""
+    return 1 if str(h.get("resblock", "1")) == "1" else 2
+
+
+def resblock_dilations(h):
+    """Dilations per ResBlock: ResBlock2 (models.py:73-83) builds its two convs from dilation[0] and dilation[1] and
+    ignores further entries."""
+    rds = [list(d) for d in h["resblock_dilation_sizes"]]
+    if resblock_type(h) == 1:
+        return rds
+    for d in rds:
+        if len(d) < 2:
+            raise ValueError("ResBlock2 needs two dilations per kernel, got %r" % (d,))
+    return [d[:2] for d in rds]
+
+
+def resblock_keys(h):
+    """ResBlock conv names per module list, in the order the native generator takes them ([stage * num_kernels + j][m]):
+    {"convs1": [...], "convs2": [...]} for ResBlock1, {"convs": [...]} for ResBlock2 (resblocks.{n}.convs.{m})."""
+    nk, ns = len(h["resblock_kernel_sizes"]), len(h["upsample_rates"])
+    nd = len(resblock_dilations(h)[0])
+    idx = [(i * nk + j, m) for i in range(ns) for j in range(nk) for m in range(nd)]
+    names = ("convs1", "convs2") if resblock_type(h) == 1 else ("convs",)
+    return {c: ["resblocks.%d.%s.%d" % (n, c, m) for n, m in idx] for c in names}
+
+
+def state_dict_keys(h, has_source=True):
+    """Every weight-norm-folded key the native generator reads."""
+    ns = len(h["upsample_rates"])
+    keys = ["conv_pre.weight", "conv_pre.bias", "conv_post.weight", "conv_post.bias"]
+    keys += ["ups.%d.%s" % (i, p) for i in range(ns) for p in ("weight", "bias")]
+    if has_source:
+        keys += ["m_source.l_linear.weight", "m_source.l_linear.bias"]
+        keys += ["noise_convs.%d.%s" % (i, p) for i in range(ns) for p in ("weight", "bias")]
+    for names in resblock_keys(h).values():
+        keys += [n + p for n in names for p in (".weight", ".bias")]
+    return keys
+
+
 class Generator:
     def __init__(self, h, state_dict=None, device="cuda"):
         self.h = h if isinstance(h, AttrDict) else AttrDict(h)
@@ -78,14 +119,18 @@ class Generator:
 
     def _build(self):
         self.release()
+        h, sd = self.h, self._sd
+        rb = resblock_type(h)
+        if rb == 2:      # name what is missing, as the reference's load_state_dict(strict=True) would
+            missing = [k for k in state_dict_keys(h, "m_source.l_linear.weight" in sd) if k not in sd]
+            if missing:
+                raise KeyError("Missing key(s) in state_dict: %s" % ", ".join('"%s"' % k for k in missing))
         lib = _lib.load()
         if not torch.cuda.is_available() or lib.dsvc_device_count() == 0:
             raise _lib.DsvcError("diffsvc_b200 NSF-HiFiGAN needs an sm_100 (B200) device: there is no CPU fallback")
-        h, sd = self.h, self._sd
-        if str(h.get("resblock", "1")) != "1":
-            raise NotImplementedError("only resblock '1' (ResBlock1) generators are supported")
         nk, ns = self.num_kernels, self.num_upsamples
-        nd = len(h.resblock_dilation_sizes[0])
+        dil = resblock_dilations(h)
+        nd = len(dil[0])
         cfg = _lib.NsfConfig()
         cfg.num_mels, cfg.sampling_rate = int(h.num_mels), int(h.sampling_rate)
         cfg.upsample_initial_channel, cfg.num_upsamples = int(h.upsample_initial_channel), ns
@@ -97,9 +142,9 @@ class Generator:
         cfg.has_source = 1 if self.has_source else 0
         for j in range(nk):
             cfg.resblock_kernel_sizes[j] = int(h.resblock_kernel_sizes[j])
-            assert len(h.resblock_dilation_sizes[j]) == nd
+            assert len(dil[j]) == nd
             for m in range(nd):
-                cfg.resblock_dilation_sizes[j][m] = int(h.resblock_dilation_sizes[j][m])
+                cfg.resblock_dilation_sizes[j][m] = int(dil[j][m])
         keep = []
 
         def f(k):
@@ -121,16 +166,16 @@ class Generator:
             w.noise_convs_b = fa(["noise_convs.%d.bias" % i for i in range(ns)])
         w.conv_pre_w, w.conv_pre_b = f("conv_pre.weight"), f("conv_pre.bias")
         w.ups_w, w.ups_b = fa(["ups.%d.weight" % i for i in range(ns)]), fa(["ups.%d.bias" % i for i in range(ns)])
-        idx = [(i * nk + j, m) for i in range(ns) for j in range(nk) for m in range(nd)]
-        w.convs1_w = fa(["resblocks.%d.convs1.%d.weight" % im for im in idx])
-        w.convs1_b = fa(["resblocks.%d.convs1.%d.bias" % im for im in idx])
-        w.convs2_w = fa(["resblocks.%d.convs2.%d.weight" % im for im in idx])
-        w.convs2_b = fa(["resblocks.%d.convs2.%d.bias" % im for im in idx])
+        # ResBlock1: convs1 / convs2; ResBlock2: resblocks.{n}.convs.{m} in the convs1 slots, convs2 stays NULL
+        first, *second = resblock_keys(h).values()
+        w.convs1_w, w.convs1_b = fa([n + ".weight" for n in first]), fa([n + ".bias" for n in first])
+        if second:
+            w.convs2_w, w.convs2_b = fa([n + ".weight" for n in second[0]]), fa([n + ".bias" for n in second[0]])
         w.conv_post_w, w.conv_post_b = f("conv_post.weight"), f("conv_post.bias")
         hd = C.c_void_p()
         dev = self.device if self.device.type == "cuda" else torch.device("cuda")
         with torch.cuda.device(dev):
-            _lib.check(lib.dsvc_nsf_create(C.byref(hd), C.byref(cfg), C.byref(w), _lib.current_stream()))
+            _lib.check(lib.dsvc_nsf_create_ex(C.byref(hd), C.byref(cfg), rb, C.byref(w), _lib.current_stream()))
         self._h = hd
 
     def forward_mel(self, mel, f0, mel_scale=1.0, rand_ini=None, sine_noise=None, seed=None):

@@ -155,7 +155,7 @@ int dsvc_diffnet_run_layer(dsvc_diffnet_t* h, int32_t layer, int32_t part, int32
 /* ------------------------------------------------------------------------------------------
  * NSF-HiFiGAN generator
  * replaces modules/nsf_hifigan/models.py:325-387 (Generator), :148-323 (SineGen,
- * SourceModuleHnNSF), :33-64 (ResBlock1), called from network/vocoders/nsf_hifigan.py:36-45,:62-72.
+ * SourceModuleHnNSF), :33-64 (ResBlock1), :73-94 (ResBlock2), called from network/vocoders/nsf_hifigan.py:36-45,:62-72.
  * ---------------------------------------------------------------------------------------- */
 typedef struct dsvc_nsf dsvc_nsf_t;
 
@@ -172,7 +172,7 @@ typedef struct {
   int32_t upsample_kernel_sizes[DSVC_NSF_MAX_STAGES];
   int32_t num_kernels;                                     /* len(h.resblock_kernel_sizes) */
   int32_t resblock_kernel_sizes[DSVC_NSF_MAX_KERNELS];
-  int32_t num_dilations;                                   /* dilations per ResBlock1 (3) */
+  int32_t num_dilations;                                   /* dilations per ResBlock1 (3); 2 for ResBlock2 */
   int32_t resblock_dilation_sizes[DSVC_NSF_MAX_KERNELS][DSVC_NSF_MAX_DILATIONS];
   int32_t harmonic_num;                                    /* 8 (models.py:334) */
   int32_t has_source;                                      /* 1: m_source + noise_convs weights are given (NSF);
@@ -199,8 +199,15 @@ typedef struct {
   const float* conv_post_b;
 } dsvc_nsf_weights;
 
+/* Generator(h) with h.resblock == '1' + load_state_dict: dsvc_nsf_create_ex(out, cfg, 1, w, stream). */
 int dsvc_nsf_create(dsvc_nsf_t** out, const dsvc_nsf_config* cfg, const dsvc_nsf_weights* w,
                     void* stream);
+/* resblock: 1 = ResBlock1 (models.py:33-70), 2 = ResBlock2 (models.py:73-94; modules/hifigan/hifigan.py:70-91),
+ * chosen as at models.py:337 / hifigan.py:119.  For 2: num_dilations must be 2 (ResBlock2 builds its two convs from
+ * dilation[0] and dilation[1]), convs1_w / convs1_b carry resblocks.{n}.convs.{m} (indexed [stage*num_kernels + j][m]),
+ * convs2_* must be NULL. */
+int dsvc_nsf_create_ex(dsvc_nsf_t** out, const dsvc_nsf_config* cfg, int32_t resblock,
+                       const dsvc_nsf_weights* w, void* stream);
 void dsvc_nsf_destroy(dsvc_nsf_t* h);
 
 /* Generator.forward(x, f0) (models.py:361-387); also HifiGanGenerator.forward(x, f0=None) of the 24 kHz

@@ -18,6 +18,10 @@ NSF_H_44K = dict(  # assumed openvpi 44.1 kHz topology (SURVEY.md section 8c): n
     n_fft=2048, win_size=2048, hop_size=512, fmin=40, fmax=16000)
 
 
+NSF_H_44K_V3 = dict(  # a HiFi-GAN "V3"-style 44.1 kHz NSF generator: ResBlock2 blocks, dilations up to 12
+    NSF_H_44K, resblock="2", resblock_kernel_sizes=[3, 5, 7], resblock_dilation_sizes=[[1, 2], [2, 6], [3, 12]])
+
+
 def synth_diffnet_weights(M=128, C=384, H=256, L=20, seed=1234):
     """Seeded synthetic DiffNet state dict with the reference's key names and init statistics
     (kaiming-normal convs net.py:47-50, default Linear init), and a NON-zero output_projection
@@ -102,3 +106,11 @@ def synth_f0(B, T, seed=11):
     f0 = f0.clamp(80.0, 800.0)
     run = (torch.sin(t * 0.05 + 3 * ph) > 0.6)      # unvoiced runs, ~20 % of frames
     return torch.where(run, torch.zeros_like(f0), f0)
+
+
+def synth_nsf_resblock2_weights(h, seed=4321):
+    """ResBlock2 ("resblock": "2") generator weights: synth_nsf_weights of the same topology with the first two
+    dilations of every list, each block's convs1.{m} renamed to convs.{m} (ResBlock2's key names, models.py:76-81)
+    and convs2 dropped."""
+    h1 = dict(h, resblock="1", resblock_dilation_sizes=[list(d)[:2] for d in h["resblock_dilation_sizes"]])
+    return {k.replace(".convs1.", ".convs."): v for k, v in synth_nsf_weights(h1, seed).items() if ".convs2." not in k}
