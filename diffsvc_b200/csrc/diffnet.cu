@@ -8,6 +8,8 @@
 #include "tc_layer.cuh"
 #include "tc_step.cuh"
 
+#include <algorithm>
+#include <climits>
 #include <cmath>
 #include <memory>
 
@@ -173,6 +175,8 @@ struct dsvc_diffnet {
   DevBuf X, S, XS, hist, CP, cond_cl, lengths, state;
   PlaneBuf Y, Z, SP, R, XIN;
   PlaneBuf Y2;           // fused-layer mode (tc_layer.cuh): conv-input plane of the odd layers (Y holds the even ones)
+  PlaneBuf Z2;           // deferred-skip schedule: gated-activation plane of the odd layers (Z holds the even ones)
+  bool skip_defer = false;   // layer l's skip half runs in layer l+1's conv kernel (enqueue_layer_conv); set in prepare
   bool pingpong = false; // Y / Y2 alternate by layer parity: a layer's out-proj never overwrites the plane its conv reads
   int fused_usable = 0;  // how many clusters of 2C/64 CTAs of tc_layer_kernel fit the device at once (probed in prepare; 0: none)
   TcMaps maps;           // TMA descriptors of the tcgen05 path (rebuilt in prepare)
@@ -294,6 +298,10 @@ static int build(dsvc_diffnet* h, const dsvc_diffnet_weights* w, cudaStream_t s)
   return DSVC_OK;
 }
 
+// the gated-activation plane layer l writes: Z, or with the deferred skip Z / Z2 by layer parity -- layer l+1's conv kernel
+// writes its own while the skip CTAs of layer l still read layer l's
+static const PlaneBuf& zplane(const dsvc_diffnet* h, int l) { return (h->skip_defer && (l & 1)) ? h->Z2 : h->Z; }
+
 // TMA descriptors of every contraction of the tcgen05 path (depend on B, Tmax and the workspace)
 static int tc_build_maps(dsvc_diffnet* h) {
   const int M = h->cfg.mel_bins, C = h->cfg.residual_channels, L = h->cfg.residual_layers;
@@ -317,7 +325,7 @@ static int tc_build_maps(dsvc_diffnet* h) {
   for (int l = 0; l < L; ++l) {
     const PlaneBuf& yin = (h->pingpong && (l & 1)) ? h->Y2 : h->Y;
     DSVC_TRY(gemm(h->maps.dil[l], yin, C, *h->h_dil[l], 3 * 2 * C));
-    DSVC_TRY(gemm(h->maps.out[l], h->Z, C, *h->h_out[l], 2 * C));
+    DSVC_TRY(gemm(h->maps.out[l], zplane(h, l), C, *h->h_out[l], 2 * C));
   }
   return DSVC_OK;
 }
@@ -357,7 +365,7 @@ static EpiInProj::Params mk_inproj(const dsvc_diffnet* h, int tsel) {
 static EpiGate::Params mk_gate(const dsvc_diffnet* h, int l) {
   const int C = h->cfg.residual_channels;
   EpiGate::Params e{};
-  e.CP = h->CP.as<float>() + (size_t)l * h->B * h->Tmax * 2 * C; e.Z = h->Z.view(h->tc); e.Tmax = h->Tmax; e.C = C;
+  e.CP = h->CP.as<float>() + (size_t)l * h->B * h->Tmax * 2 * C; e.Z = zplane(h, l).view(h->tc); e.Tmax = h->Tmax; e.C = C;
   e.fast = h->tc ? 1 : 0; e.wscale = h->tc ? h->h_dil[l]->inv_scale : 1.f;
   return e;
 }
@@ -390,13 +398,26 @@ static EpiHead::Params mk_head(const dsvc_diffnet* h, const HeadArgs& ha) {
   return e;
 }
 
-// K3a: dilated conv + hoisted conditioner + gate -> Z
-static int enqueue_layer_conv(dsvc_diffnet* h, int l, cudaStream_t s) {
+// K0: input projection + ReLU
+static int enqueue_inproj(dsvc_diffnet* h, int tsel, cudaStream_t s) {
+  const int M = h->cfg.mel_bins, C = h->cfg.residual_channels;
+  const EpiInProj::Params e = mk_inproj(h, tsel);
+  if (h->tc) return tc_launch<EpiInProj>(h->maps.in, e, h->B, h->Tmax, M, C, 1, 0, h->passes, s, tiles_of(h));
+  return launch_fp32<EpiInProj>(h, base_params(h->XIN.f32.as<float>(), h->w_in.as<float>(), h->B, h->Tmax, M, C, 1, 0), e, s);
+}
+
+// K3a: dilated conv + hoisted conditioner + gate -> Z.  With the deferred skip (skip_defer_pick) the same grid also runs
+// the skip half of layer l-1's output projection: 64-wide out-projection tiles C/64 .. 2C/64-1, in block rows behind the
+// conv's 2C/64.  Nothing in layer l waits for them: they read Z_{l-1} and S, written two launches back.
+static int enqueue_layer_conv(dsvc_diffnet* h, int l, int tsel, cudaStream_t s) {
   const int C = h->cfg.residual_channels, B = h->B, T = h->Tmax;
   const int dil = 1 << (l % h->cfg.dilation_cycle_length);
   const EpiGate::Params e = mk_gate(h, l);
   if (h->tc) {
     const TcGemmMaps& m = h->maps.dil[l];
+    if (h->skip_defer && l > 0)
+      return tc_pair2_launch_bn<EpiGate, EpiOutProj, 64>(m, e, C, 2 * C, 3, dil, 2 * C / 64, h->maps.out[l - 1],
+                                                          mk_outproj(h, l - 1, tsel), C, 2 * C, 1, 0, C / 64, C / 64, B, T, s);
     // grids that leave SMs idle (one clip): one tap per CTA in a 3-CTA cluster, reduced through an L2 slab
     // (measured, 43 frames: CTA pairs 295 us per step, split-K + pairs 316, split-K + single-CTA kernels 328 -- so the
     //  split is automatic only next to the single-CTA kernels, and on request: DSVC_SPLITK >= 1)
@@ -411,13 +432,22 @@ static int enqueue_layer_conv(dsvc_diffnet* h, int l, cudaStream_t s) {
   return launch_fp32<EpiGate>(h, base_params(h->Y.f32.as<float>(), W, B, T, C, 2 * C, 3, dil), e, s);
 }
 
-// K3b: output projection + residual + skip
+// K3b: output projection + residual + skip.  With the deferred skip: the residual half alone (out-projection tiles
+// 0 .. C/64-1, the same 64-wide tiles and functor as the whole projection)
 static int enqueue_layer_out(dsvc_diffnet* h, int l, int tsel, cudaStream_t s) {
   const int C = h->cfg.residual_channels, B = h->B, T = h->Tmax;
   const EpiOutProj::Params e = mk_outproj(h, l, tsel);
+  if (h->skip_defer) return tc_pair_launch_bn<EpiOutProj, 64>(h->maps.out[l], e, B, T, C, 2 * C, 1, 0, s, TcTiles{}, 0, C / 64);
   if (h->tc) return tc_launch<EpiOutProj>(h->maps.out[l], e, B, T, C, 2 * C, 1, 0, h->passes, s, tiles_of(h));
   const float* W = h->w_out.as<float>() + (size_t)l * 2 * C * C;
   return launch_fp32<EpiOutProj>(h, base_params(h->Z.f32.as<float>(), W, B, T, C, 2 * C, 1, 0), e, s);
+}
+
+// the deferred skip half of the last layer (there is no next conv kernel to carry it): S / sqrt(L) -> SP
+static int enqueue_layer_skip(dsvc_diffnet* h, int l, int tsel, cudaStream_t s) {
+  const int C = h->cfg.residual_channels;
+  return tc_pair_launch_bn<EpiOutProj, 64>(h->maps.out[l], mk_outproj(h, l, tsel), h->B, h->Tmax, C, 2 * C, 1, 0, s, TcTiles{},
+                                          C / 64, C / 64);
 }
 
 // K3a + K3b as one kernel (tc_layer.cuh): a cluster of 2C/64 CTAs per frame tile, cluster barrier between the conv
@@ -515,24 +545,41 @@ static int step_pick_bn(dsvc_diffnet* h) {
   return 0;
 }
 
+// Deferred skip (DESIGN.md 3.1d): every layer kernel pre-launches whole.  The 64-wide out-projection of one clip is
+// 2C/64 x frame-tile CTAs like the conv, and with ~206 KB of shared memory per CTA the two grids do not fit the SMs
+// together, so half of each grid could only enter as the previous kernel drained.  Its skip half is read by nobody until
+// the skip projection: it moves into the next layer's conv grid, and what stays between two convs is the residual half
+// (C/64 tiles).  Conv + residual CTAs then fit the SMs at once.  Same tiles, same functors, same order of the skip sums:
+// bit-identical to the layer-by-layer schedule.  Only the CTA-pair path with 64-wide tiles on a dense grid takes it;
+// DSVC_SKIP_DEFER=0 keeps the layer-by-layer schedule (read when the handle is prepared).
+static bool skip_defer_pick(const dsvc_diffnet* h) {
+  const char* e = getenv("DSVC_SKIP_DEFER");
+  if (e && atoi(e) == 0) return false;
+  const char* skv = getenv("DSVC_SPLITK");
+  if (skv && atoi(skv) >= 1) return false;
+  const int C = h->cfg.residual_channels;
+  if (!(h->tc && h->passes == 3 && tc_pair_enabled()) || h->tile_slots > 0 || h->step_bn > 0 || fused_layers(h)) return false;
+  if (C % 64 != 0 || tc_pick_bn(h->B, h->Tmax, 2 * C) != 64) return false;
+  const long long ft = (long long)tc_pair_frame_ctas(h->Tmax) * h->B;
+  return ft * (2 * C / 64) + ft * (C / 64) <= h->num_sms;
+}
+
 // one denoiser evaluation: enqueue all kernels on `s`
 static int enqueue_eval(dsvc_diffnet* h, const HeadArgs& ha, cudaStream_t s) {
   const int M = h->cfg.mel_bins, C = h->cfg.residual_channels, L = h->cfg.residual_layers;
   const int B = h->B, T = h->Tmax;
   if (h->step_bn > 0) return enqueue_eval_step(h, ha, s);
-  {  // K0 input_projection + ReLU
-    const EpiInProj::Params e = mk_inproj(h, ha.tsel);
-    if (h->tc) DSVC_TRY(tc_launch<EpiInProj>(h->maps.in, e, B, T, M, C, 1, 0, h->passes, s, tiles_of(h)));
-    else DSVC_TRY(launch_fp32<EpiInProj>(h, base_params(h->XIN.f32.as<float>(), h->w_in.as<float>(), B, T, M, C, 1, 0), e, s));
-  }
+  DSVC_TRY(enqueue_inproj(h, ha.tsel, s));
   for (int l = 0; l < L; ++l) {
     if (fused_layers(h)) {
       DSVC_TRY(enqueue_layer_fused(h, l, ha.tsel, s));
       continue;
     }
-    DSVC_TRY(enqueue_layer_conv(h, l, s));
-    DSVC_TRY(enqueue_layer_out(h, l, ha.tsel, s));
+    DSVC_TRY(enqueue_layer_conv(h, l, ha.tsel, s));
+    // deferred skip: the last layer's residual output x' is read by nobody (skip projection and head read SP / R / XS)
+    if (!h->skip_defer || l + 1 < L) DSVC_TRY(enqueue_layer_out(h, l, ha.tsel, s));
   }
+  if (h->skip_defer) DSVC_TRY(enqueue_layer_skip(h, L - 1, ha.tsel, s));
   {  // K4a skip_projection + ReLU
     const EpiSkipProj::Params e = mk_skip(h);
     if (h->tc) DSVC_TRY(tc_launch<EpiSkipProj>(h->maps.skip, e, B, T, C, C, 1, 0, h->passes, s, tiles_of(h)));
@@ -732,10 +779,6 @@ int dsvc_diffnet_prepare(dsvc_diffnet_t* h, int32_t B, int32_t Tmax, const int32
     h->tile_slots = h->tile_live = 0;
   }
   DSVC_CUDA(cudaStreamSynchronize(s));   // `len` / `tab` are stack-owned staging buffers
-  if (resized || !h->prepared || ragged_changed) {
-    h->g_ddpm_valid = h->g_plms_valid = false;
-    if (tc) DSVC_TRY(tc_build_maps(h));
-  }
   {
     const int bn = step_pick_bn(h);
     if (bn != h->step_bn) h->g_ddpm_valid = h->g_plms_valid = false;
@@ -745,6 +788,13 @@ int dsvc_diffnet_prepare(dsvc_diffnet_t* h, int32_t B, int32_t Tmax, const int32
       DSVC_TRY(h->step_flags.reserve(fb));
       DSVC_CUDA(cudaMemsetAsync(h->step_flags.p, 0, fb, s));      // both counter sets and the sequence word start at 0
     }
+  }
+  const bool defer = skip_defer_pick(h);        // the Z planes the maps point at depend on it
+  if (defer) DSVC_TRY(h->Z2.reserve(n * C, tc));
+  if (resized || !h->prepared || ragged_changed || defer != h->skip_defer) {
+    h->g_ddpm_valid = h->g_plms_valid = false;
+    h->skip_defer = defer;
+    if (tc) DSVC_TRY(tc_build_maps(h));
   }
   // cond [B][H][T] -> channels-last, then all L conditioner projections in one GEMM
   {
@@ -793,7 +843,7 @@ int dsvc_cond_encode(const float* hubert, const int64_t* mel2ph, const float* f0
 int dsvc_diffnet_run_layer(dsvc_diffnet_t* h, int32_t layer, int32_t part, int32_t iters, void* stream) {
   DSVC_REQUIRE(h, "dsvc_diffnet_run_layer: null handle");
   if (!h->prepared) { set_error("dsvc_diffnet_run_layer: call dsvc_diffnet_prepare first"); return DSVC_ESTATE; }
-  DSVC_REQUIRE(layer >= 0 && layer < h->cfg.residual_layers && part >= 0 && part <= 3 && iters >= 0, "bad layer/part/iters");
+  DSVC_REQUIRE(layer >= 0 && layer < h->cfg.residual_layers && part >= 0 && part <= 4 && iters >= 0, "bad layer/part/iters");
   if (part == 3) {
     // developer probe: `iters` whole evaluations through the step kernel; a -DDSVC_TIMELINE build prints its phase stamps
     if (h->step_bn == 0) { set_error("dsvc_diffnet_run_layer: part 3 needs the step kernel (tc_step.cuh) for this shape"); return DSVC_ESTATE; }
@@ -840,6 +890,66 @@ int dsvc_diffnet_run_layer(dsvc_diffnet_t* h, int32_t layer, int32_t part, int32
 #endif
     return DSVC_OK;
   }
+  if (part == 4) {
+    // developer probe: layer `layer`'s two kernels in the alternation of a real evaluation.  Run 0 enqueues the evaluation
+    // up to that layer's conv kernel, run 1 up to its out-projection; a -DDSVC_TIMELINE build prints the stamps of the
+    // kernel each run ends with.
+    if (!h->tc || h->step_bn > 0 || fused_layers(h)) {
+      set_error("dsvc_diffnet_run_layer: part 4 needs the per-layer tensor-core kernels");
+      return DSVC_ESTATE;
+    }
+    cudaStream_t s4 = (cudaStream_t)stream;
+    for (int run = 0; run < 2; ++run) {
+      set_state_kernel<<<1, 1, 0, s4>>>(h->state.as<StepState>(), 500, 1, 1ull, nullptr);
+      DSVC_LAUNCH_CHECK();
+      DSVC_TRY(enqueue_inproj(h, 0, s4));
+      for (int l = 0; l <= layer; ++l) {
+        DSVC_TRY(enqueue_layer_conv(h, l, 0, s4));
+        if (l < layer || run == 1) DSVC_TRY(enqueue_layer_out(h, l, 0, s4));
+      }
+#ifdef DSVC_TIMELINE
+      static long long tl4[1024][16];
+      DSVC_CUDA(cudaStreamSynchronize(s4));
+      DSVC_CUDA(cudaMemcpyFromSymbol(tl4, g_timeline, sizeof(tl4)));
+      const int C = h->cfg.residual_channels, gx = tc_pair_frame_ctas(h->Tmax), bn = tc_pick_bn(h->B, h->Tmax, 2 * C);
+      // block rows of the kernel and the role of each: 0 gate, 1 skip half, 2 out-projection (residual half when deferred)
+      const int n_conv = 2 * C / bn, n_skip = (h->skip_defer && layer > 0) ? C / 64 : 0;
+      const int rows = run == 0 ? n_conv + n_skip : (h->skip_defer ? C / 64 : 2 * C / bn);
+      const int nct = gx * rows * h->B;
+      if (nct > 1024) { printf("part 4: %d CTAs, more than the timeline holds\n", nct); continue; }
+      auto role = [&](int c) { const int y = (c / gx) % rows; return run == 1 ? 2 : (y < n_conv ? 0 : 1); };
+      long long e0 = tl4[0][15], rel = tl4[0][13];
+      for (int c = 0; c < nct; ++c) { e0 = std::min(e0, tl4[c][15]); rel = std::min(rel, tl4[c][13]); }
+      const char* names[3] = {"gate", "skip", "out"};
+      printf("timeline part 4, layer %d, %s kernel (%s schedule), %d CTAs; ns after the first CTA entry; release = the earliest "
+             "return from griddepcontrol.wait (%lld)\n", layer, run == 0 ? "conv" : "out-projection",
+             h->skip_defer ? "deferred-skip" : "layer-by-layer", nct, rel - e0);
+      // a CTA that was resident and waiting leaves griddepcontrol.wait at the release; one that entered as the previous
+      // kernel drained reaches it only after its own set-up (barrier init, TMEM alloc, weight prefetch: ~1-2 us)
+      for (int r = 0; r < 3; ++r) {
+        int n = 0, waiting = 0;
+        long long last_in = 0, first_done = LLONG_MAX, last_done = 0, last_ops = 0;
+        for (int c = 0; c < nct; ++c) {
+          if (role(c) != r) continue;
+          ++n;
+          waiting += tl4[c][13] - rel < 500;
+          last_in = std::max(last_in, tl4[c][15] - e0);
+          first_done = std::min(first_done, tl4[c][14] - e0);
+          last_done = std::max(last_done, tl4[c][14] - e0);
+          last_ops = std::max(last_ops, tl4[c][13] - e0);
+        }
+        if (n == 0) continue;
+        printf("  %-4s %3d CTAs: %3d waiting at the release (past the wait < 0.5 us after it) | last entry %6lld | last past the wait "
+               "%6lld | done %6lld .. %6lld\n", names[r], n, waiting, last_in, last_ops, first_done, last_done);
+      }
+      for (int c = 0; c < nct; c += 2)
+        printf("  cta %3d %-4s: entry %6lld | past wait %6lld | first operands +%5lld cyc | done %6lld\n", c, names[role(c)],
+               tl4[c][15] - e0, tl4[c][13] - e0, tl4[c][1], tl4[c][14] - e0);
+      fflush(stdout);
+#endif
+    }
+    return DSVC_OK;
+  }
   if (part == 2 && !fused_layers(h)) {
     set_error("dsvc_diffnet_run_layer: part 2 (fused layer kernel) needs DSVC_FUSED_LAYER and a tensor-core handle whose "
               "2C/64 channel tiles form a schedulable cluster");
@@ -849,7 +959,7 @@ int dsvc_diffnet_run_layer(dsvc_diffnet_t* h, int32_t layer, int32_t part, int32
   set_state_kernel<<<1, 1, 0, s>>>(h->state.as<StepState>(), 0, 1, 0ull, nullptr);   // a valid step-table row
   DSVC_LAUNCH_CHECK();
   for (int i = 0; i < iters; ++i) {
-    if (part == 0) DSVC_TRY(enqueue_layer_conv(h, layer, s));
+    if (part == 0) DSVC_TRY(enqueue_layer_conv(h, layer, 0, s));
     else if (part == 1) DSVC_TRY(enqueue_layer_out(h, layer, 0, s));
     else DSVC_TRY(enqueue_layer_fused(h, layer, 0, s));
   }

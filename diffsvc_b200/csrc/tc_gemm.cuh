@@ -264,9 +264,13 @@ __device__ long long g_timeline[1024][16];
 // slot 15: %globaltimer (ns) at CTA entry -- the one clock all CTAs share: orders early (pre-launched) and late CTAs
 #define TL_ENTRY() do { if (threadIdx.x == 0) { unsigned long long gt_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt_)); \
   g_timeline[((blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) & 1023][15] = (long long)gt_; } } while (0)
+// %globaltimer (ns) into `slot` by thread 0 (the pair kernel: 13 = past griddepcontrol.wait, 14 = epilogue done)
+#define TL_GT(slot) do { if (threadIdx.x == 0) { unsigned long long gt_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt_)); \
+  g_timeline[((blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) & 1023][slot] = (long long)gt_; } } while (0)
 #else
 #define TL_MARK(slot) do { } while (0)
 #define TL_ENTRY() do { } while (0)
+#define TL_GT(slot) do { } while (0)
 #endif
 
 // ===== epilogue (all 16 warps): TMEM -> registers -> smem transpose -> fused functor -> global =====

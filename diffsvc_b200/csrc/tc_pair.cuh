@@ -73,12 +73,12 @@ __device__ __forceinline__ void umma2_commit_both(uint32_t bar) {
                ::"r"(bar), "h"((uint16_t)3) : "memory");
 }
 
+// One CTA of a pair: ny is the channel-tile index of its tile (the block row of tc_pair_kernel, the role-adjusted row of
+// tc_pair2_kernel).  The tensor maps are the kernel's __grid_constant__ parameters, passed by reference.
 template <class Epi, int BN>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-tc_pair_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
-               const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl,
-               const typename Epi::Params ep, int T, int K, int N, int taps, int dil, const int2* __restrict__ tiles) {
-#if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ >= 1000)
+__device__ __forceinline__ void tc_pair_cta(const CUtensorMap& tmAh, const CUtensorMap& tmAl, const CUtensorMap& tmBh,
+                                            const CUtensorMap& tmBl, const typename Epi::Params& ep, int T, int K, int N,
+                                            int taps, int dil, const int2* __restrict__ tiles, int ny) {
   using Cfg = TcPairCfg<BN>;
   constexpr int STAGES = Cfg::STAGES;
   constexpr int H = Cfg::H;
@@ -149,10 +149,10 @@ tc_pair_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
       // simply holds ITS half of the tile's rows, hi block then lo block: P = [ wh_half (128 rows) ; wl_half (128 rows) ]
       int r0, r1;                                     // two 64-row boxes
       if constexpr (Epi::kPair) {                     // [128 gate | 128 filter] from two packed super-tiles
-        const int sb = tap * N + (int)blockIdx.y * 256;
+        const int sb = tap * N + ny * 256;
         r0 = sb + (rank == 0 ? 0 : 64); r1 = r0 + 128;
       } else {
-        r0 = tap * N + (int)blockIdx.y * 256 + (int)rank * 128; r1 = r0 + 64;
+        r0 = tap * N + ny * 256 + (int)rank * 128; r1 = r0 + 64;
       }
       const uint32_t bar = full_bar_leader(s);
       const uint32_t p = tile_p(s);
@@ -166,10 +166,10 @@ tc_pair_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
       // gate|filter packing: a 128-row super-tile holds [64 gate rows | 64 filter rows]; a BN-wide tile takes
       // H gate rows and the matching H filter rows
       const int per = 128 / BN;                       // tiles per super-tile (BN = 64: 2, BN = 128: 1)
-      ra = tap * N + (int)(blockIdx.y / per) * 128 + (int)(blockIdx.y % per) * H;
+      ra = tap * N + (ny / per) * 128 + (ny % per) * H;
       rb = ra + 64;
     } else {
-      ra = tap * N + (int)blockIdx.y * BN;
+      ra = tap * N + ny * BN;
       rb = ra + H;
     }
     const uint32_t bar = full_bar_leader(s);
@@ -199,6 +199,7 @@ tc_pair_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
     }
     __syncwarp();
     pdl_wait();                                               // activations were written by the previous kernel
+    TL_GT(13);
     if (elect_one_sync()) {
       for (int it = 0; it < pre; ++it) load_a(it, it);
     }
@@ -251,18 +252,49 @@ tc_pair_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
   }
   pdl_wait();
 #ifdef DSVC_TIMELINE
-  tc_epilogue<Epi, BN>(ep, smem_raw, smem_base, tmem_base, tmem_full_bar, 0u, T, N, m0, (int)blockIdx.y, b, warp, lane, true, tl0, 0, BN == 256 ? 0 : H);
+  tc_epilogue<Epi, BN>(ep, smem_raw, smem_base, tmem_base, tmem_full_bar, 0u, T, N, m0, ny, b, warp, lane, true, tl0, 0, BN == 256 ? 0 : H);
 #else
-  tc_epilogue<Epi, BN>(ep, smem_raw, smem_base, tmem_base, tmem_full_bar, 0u, T, N, m0, (int)blockIdx.y, b, warp, lane, true, BN == 256 ? 0 : H);
+  tc_epilogue<Epi, BN>(ep, smem_raw, smem_base, tmem_base, tmem_full_bar, 0u, T, N, m0, ny, b, warp, lane, true, BN == 256 ? 0 : H);
 #endif
   if (warp == 4) TL_MARK(6);
   tc_fence_before();
   __syncthreads();
+  TL_GT(14);
   cluster_sync_all();                   // both CTAs have drained their accumulator halves
   if (warp == 2) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(2 * BN) : "memory");
   }
+}
+
+// Channel tiles ny0 .. ny0 + gridDim.y - 1 of an N-wide contraction (ny0 > 0: the second half of the WaveNet
+// out-projection, launched on its own after the last layer)
+template <class Epi, int BN>
+__global__ void __launch_bounds__(TC_THREADS, 1)
+tc_pair_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
+               const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl,
+               const typename Epi::Params ep, int T, int K, int N, int taps, int dil, const int2* __restrict__ tiles, int ny0) {
+#if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ >= 1000)
+  tc_pair_cta<Epi, BN>(tmAh, tmAl, tmBh, tmBl, ep, T, K, N, taps, dil, tiles, ny0 + (int)blockIdx.y);
+#endif
+}
+
+// Two independent contractions of one frame range in one grid (dense layout, no tile table): block rows y < nA run
+// role A (channel tiles 0 .. nA - 1 of its N), rows y >= nA role B (channel tiles nyB + y - nA of its N).  Each role has
+// its own tensor maps, epilogue, K, taps and dilation; the branch is uniform per CTA pair.  Both roles keep the PDL
+// protocol of the plain kernel (dependents released at entry, griddepcontrol.wait before the first activation load), so
+// role B may read what the kernel two launches back wrote: the previous kernel completes only after its own wait.
+template <class EpiA, class EpiB, int BN>
+__global__ void __launch_bounds__(TC_THREADS, 1)
+tc_pair2_kernel(const __grid_constant__ CUtensorMap aAh, const __grid_constant__ CUtensorMap aAl,
+                const __grid_constant__ CUtensorMap aBh, const __grid_constant__ CUtensorMap aBl,
+                const typename EpiA::Params epA, int KA, int NA, int tapsA, int dilA, int nA,
+                const __grid_constant__ CUtensorMap bAh, const __grid_constant__ CUtensorMap bAl,
+                const __grid_constant__ CUtensorMap bBh, const __grid_constant__ CUtensorMap bBl,
+                const typename EpiB::Params epB, int KB, int NB, int tapsB, int dilB, int nyB, int T) {
+#if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ >= 1000)
+  if ((int)blockIdx.y < nA) tc_pair_cta<EpiA, BN>(aAh, aAl, aBh, aBl, epA, T, KA, NA, tapsA, dilA, nullptr, (int)blockIdx.y);
+  else tc_pair_cta<EpiB, BN>(bAh, bAl, bBh, bBl, epB, T, KB, NB, tapsB, dilB, nullptr, nyB + (int)blockIdx.y - nA);
 #endif
 }
 
@@ -272,28 +304,61 @@ inline bool tc_pair_enabled() {
   return !(e && atoi(e) == 0);
 }
 
+// frame tiles in pairs (an odd last one pairs with an empty tile): the grid's x extent of a dense layout
+inline int tc_pair_frame_ctas(int T) { return 2 * ceil_div(ceil_div(T, TC_BM), 2); }
+
+// cluster of two CTAs along x, programmatic dependent launch
+struct TcPairLaunch {
+  cudaLaunchConfig_t cfg{};
+  cudaLaunchAttribute attr[2];
+  TcPairLaunch(dim3 grid, int smem, cudaStream_t s) {
+    cfg.gridDim = grid;
+    cfg.blockDim = dim3(TC_THREADS);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[1].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 2;
+  }
+};
+
+// the weight maps of a BN-wide pair tile: boxes of H rows (BN = 256: two 64-row boxes per half)
+template <int BN> const CUtensorMap& tc_pair_bh(const TcGemmMaps& m) { return BN == 64 ? m.b32_hi : m.b64_hi; }
+template <int BN> const CUtensorMap& tc_pair_bl(const TcGemmMaps& m) { return BN == 64 ? m.b32_lo : m.b64_lo; }
+
+// channel tiles ny0 .. ny0 + n_ny - 1 (n_ny = 0: all N / BN)
 template <class Epi, int BN>
 int tc_pair_launch_bn(const TcGemmMaps& m, const typename Epi::Params& e, int B, int T, int K, int N, int taps, int dil,
-                      cudaStream_t s, TcTiles tt = TcTiles{}) {
+                      cudaStream_t s, TcTiles tt = TcTiles{}, int ny0 = 0, int n_ny = 0) {
   DSVC_TRY((ensure_dyn_smem<tc_pair_kernel<Epi, BN>>(TcPairCfg<BN>::SMEM)));
-  cudaLaunchConfig_t cfg{};
-  // frame tiles in pairs (an odd last one pairs with an empty tile); a ragged batch's table has an even slot count
-  cfg.gridDim = tt.tab ? dim3(tt.slots, N / BN, 1) : dim3(2 * ceil_div(ceil_div(T, TC_BM), 2), N / BN, B);
-  cfg.blockDim = dim3(TC_THREADS);
-  cfg.dynamicSmemBytes = TcPairCfg<BN>::SMEM;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  const CUtensorMap& bh = (BN == 64) ? m.b32_hi : m.b64_hi;      // boxes of H rows (BN = 256: two 64-row boxes per half)
-  const CUtensorMap& bl = (BN == 64) ? m.b32_lo : m.b64_lo;
-  DSVC_CUDA(cudaLaunchKernelEx(&cfg, tc_pair_kernel<Epi, BN>, m.a_hi, m.a_lo, bh, bl, e, T, K, N, taps, dil, tt.tab));
+  const int ny = n_ny > 0 ? n_ny : N / BN;
+  DSVC_REQUIRE(ny0 >= 0 && ny0 + ny <= N / BN, "tc_pair_launch: channel tiles %d..%d of %d", ny0, ny0 + ny - 1, N / BN);
+  // a ragged batch's table has an even slot count
+  TcPairLaunch l(tt.tab ? dim3(tt.slots, ny, 1) : dim3(tc_pair_frame_ctas(T), ny, B), TcPairCfg<BN>::SMEM, s);
+  DSVC_CUDA(cudaLaunchKernelEx(&l.cfg, tc_pair_kernel<Epi, BN>, m.a_hi, m.a_lo, tc_pair_bh<BN>(m), tc_pair_bl<BN>(m), e, T, K, N,
+                               taps, dil, tt.tab, ny0));
+  DSVC_LAUNCH_CHECK();
+  return DSVC_OK;
+}
+
+// tc_pair2_kernel: role A = channel tiles 0 .. nA - 1 of (mA, NA), role B = tiles nyB .. nyB + nB - 1 of (mB, NB); one item
+// of T frames or a dense batch of B
+template <class EpiA, class EpiB, int BN>
+int tc_pair2_launch_bn(const TcGemmMaps& mA, const typename EpiA::Params& eA, int KA, int NA, int tapsA, int dilA, int nA,
+                       const TcGemmMaps& mB, const typename EpiB::Params& eB, int KB, int NB, int tapsB, int dilB, int nyB, int nB,
+                       int B, int T, cudaStream_t s) {
+  DSVC_TRY((ensure_dyn_smem<tc_pair2_kernel<EpiA, EpiB, BN>>(TcPairCfg<BN>::SMEM)));
+  DSVC_REQUIRE(KA % TC_BK == 0 && KB % TC_BK == 0 && nA > 0 && nA <= NA / BN && nB > 0 && nyB >= 0 && nyB + nB <= NB / BN,
+               "tc_pair2_launch: bad roles (K %d / %d, tiles %d of %d, %d..%d of %d)", KA, KB, nA, NA / BN, nyB, nyB + nB - 1, NB / BN);
+  TcPairLaunch l(dim3(tc_pair_frame_ctas(T), nA + nB, B), TcPairCfg<BN>::SMEM, s);
+  DSVC_CUDA(cudaLaunchKernelEx(&l.cfg, tc_pair2_kernel<EpiA, EpiB, BN>, mA.a_hi, mA.a_lo, tc_pair_bh<BN>(mA), tc_pair_bl<BN>(mA), eA,
+                               KA, NA, tapsA, dilA, nA, mB.a_hi, mB.a_lo, tc_pair_bh<BN>(mB), tc_pair_bl<BN>(mB), eB, KB, NB,
+                               tapsB, dilB, nyB, T));
   DSVC_LAUNCH_CHECK();
   return DSVC_OK;
 }

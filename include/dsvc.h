@@ -148,8 +148,13 @@ int dsvc_cond_encode(const float* hubert, const int64_t* mel2ph, const float* f0
 /* Measurement hook (bench.py roofline): enqueue `iters` back-to-back launches of one kernel of the
  * WaveNet layer `layer` on the prepared workspace.  part 0 = dilated conv + conditioner + gate
  * (net.py:69-77), part 1 = output projection + residual + skip (net.py:79-84), part 2 = both as the
- * one fused layer kernel (opt-in DSVC_FUSED_LAYER; DSVC_ESTATE when that mode is not active).  The workspace
- * contents afterwards are unspecified (call prepare / a sampler again before trusting results). */
+ * one fused layer kernel (opt-in DSVC_FUSED_LAYER; DSVC_ESTATE when that mode is not active).  Under the
+ * deferred-skip schedule (the default for one clip, DESIGN.md 3.1d) part 0 is the conv kernel of `layer`
+ * together with the skip half of layer `layer` - 1's output projection (the conv alone for layer 0), and
+ * part 1 is the residual half of the output projection.  part 4 = developer probe: the evaluation up to
+ * `layer`'s conv kernel, then up to its output projection (`iters` ignored; a -DDSVC_TIMELINE build
+ * prints both kernels' in-kernel stamps).  The workspace contents afterwards are unspecified (call
+ * prepare / a sampler again before trusting results). */
 int dsvc_diffnet_run_layer(dsvc_diffnet_t* h, int32_t layer, int32_t part, int32_t iters, void* stream);
 
 /* ------------------------------------------------------------------------------------------
