@@ -19,22 +19,23 @@ namespace dsvc {
 // small kernels
 // ---------------------------------------------------------------------------------------------
 
-// [B][R][Cc] (Cc contiguous) -> [B][Cc][R] tiled transpose, optional operand-plane copy of the output
-__global__ void transpose_kernel(const float* __restrict__ in, float* __restrict__ out, Plane pl, int R, int Cc) {
+// [B][R][Cc] (Cc contiguous, rows ldi apart) -> [B][Cc][R] (rows ldo apart) tiled transpose, optional operand-plane copy
+// of the output.  ldi / ldo > the logical width: the mel axis of the tensor-core path's internal state, padded to Mp
+__global__ void transpose_kernel(const float* __restrict__ in, float* __restrict__ out, Plane pl, int R, int Cc, int ldi, int ldo) {
   __shared__ float tile[32][33];
   const int b = blockIdx.z;
   const int c0 = blockIdx.x * 32, r0 = blockIdx.y * 32;
-  const float* ib = in + (size_t)b * R * Cc;
+  const float* ib = in + (size_t)b * R * ldi;
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
     const int r = r0 + i, c = c0 + threadIdx.x;
-    tile[i][threadIdx.x] = (r < R && c < Cc) ? ib[(size_t)r * Cc + c] : 0.f;
+    tile[i][threadIdx.x] = (r < R && c < Cc) ? ib[(size_t)r * ldi + c] : 0.f;
   }
   __syncthreads();
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
     const int c = c0 + i, r = r0 + threadIdx.x;
     if (c < Cc && r < R) {
       const float v = tile[threadIdx.x][i];
-      const size_t idx = ((size_t)b * Cc + c) * R + r;
+      const size_t idx = ((size_t)b * Cc + c) * ldo + r;
       if (out) out[idx] = v;
       if (pl.f32) pl.f32[idx] = v;
       if (pl.hi) {
@@ -47,10 +48,10 @@ __global__ void transpose_kernel(const float* __restrict__ in, float* __restrict
   }
 }
 
-// Packed ragged batch: the caller's [B][Cc][uT] tensor -> rows of the packed frame axis [Tp][Cc] (padding rows: zeros),
+// Packed ragged batch: the caller's [B][Cc][uT] tensor -> rows of the packed frame axis [Tp][ldo] (padding rows: zeros),
 // optional operand-plane copy.  Consecutive packed rows are consecutive frames of one item, so both sides coalesce.
 __global__ void pack_rows_kernel(const float* __restrict__ in, float* __restrict__ out, Plane pl, const int2* __restrict__ rowmap,
-                                 int Tp, int Cc, int uT) {
+                                 int Tp, int Cc, int uT, int ldo) {
   __shared__ float tile[32][33];
   const int c0 = blockIdx.y * 32, r0 = blockIdx.x * 32;
   {
@@ -66,7 +67,7 @@ __global__ void pack_rows_kernel(const float* __restrict__ in, float* __restrict
     const int r = r0 + i, c = c0 + threadIdx.x;
     if (r < Tp && c < Cc) {
       const float v = tile[threadIdx.x][i];
-      const size_t idx = (size_t)r * Cc + c;
+      const size_t idx = (size_t)r * ldo + c;
       if (out) out[idx] = v;
       if (pl.f32) pl.f32[idx] = v;
       if (pl.hi) {
@@ -79,15 +80,15 @@ __global__ void pack_rows_kernel(const float* __restrict__ in, float* __restrict
   }
 }
 
-// the way back: rows of the packed axis [Tp][Cc] -> the live frames of the caller's [B][Cc][uT] tensor (frames at or
+// the way back: rows of the packed axis [Tp][ldi] -> the live frames of the caller's [B][Cc][uT] tensor (frames at or
 // beyond an item's length keep what the caller passed in)
 __global__ void unpack_rows_kernel(const float* __restrict__ in, float* __restrict__ out, const int2* __restrict__ rowmap,
-                                   int Tp, int Cc, int uT) {
+                                   int Tp, int Cc, int uT, int ldi) {
   __shared__ float tile[32][33];
   const int c0 = blockIdx.y * 32, r0 = blockIdx.x * 32;
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
     const int r = r0 + i, c = c0 + threadIdx.x;
-    tile[i][threadIdx.x] = (r < Tp && c < Cc) ? in[(size_t)r * Cc + c] : 0.f;
+    tile[i][threadIdx.x] = (r < Tp && c < Cc) ? in[(size_t)r * ldi + c] : 0.f;
   }
   __syncthreads();
   const int r = r0 + threadIdx.x;
@@ -157,6 +158,8 @@ struct dsvc_diffnet {
   dsvc_diffnet_config cfg;
   bool tc = false;       // tcgen05 path
   int passes = 3;
+  int Mp = 0;            // row stride of the mel axis inside the library (XS, hist, XIN, h_in / h_head / b_head): mel_bins
+                         // rounded up to a whole 64-wide K block / tile on the tcgen05 path, mel_bins on the FFMA path
   // fp32 weights (GEMM layouts: [taps][Cout][Cin])
   DevBuf w_in, b_in, w_dil, w_cond, b_cond, w_out, b_out, w_skip, b_skip, w_head, b_head;
   DevBuf dtab;           // [Tn][L][C]
@@ -236,7 +239,11 @@ static int build(dsvc_diffnet* h, const dsvc_diffnet_weights* w, cudaStream_t s)
   DSVC_TRY(h->w_skip.upload(w->skip_projection_w, (size_t)C * C * 4, s));
   DSVC_TRY(h->b_skip.upload(w->skip_projection_b, (size_t)C * 4, s));
   DSVC_TRY(h->w_head.upload(w->output_projection_w, (size_t)M * C * 4, s));
-  DSVC_TRY(h->b_head.upload(w->output_projection_b, (size_t)M * 4, s));
+  // the head bias is read as float4 at every column of the (padded) head tile: [Mp], zeros past M
+  const int Mp = h->Mp;
+  std::vector<float> bh((size_t)Mp, 0.f);
+  memcpy(bh.data(), w->output_projection_b, (size_t)M * 4);
+  DSVC_TRY(upload_f(h->b_head, bh, s));
 
   // dilated convs: [2C][C][3] -> [L][tap][2C paired][C]; pairing puts, in every 128-column tile,
   // 64 gate rows next to their 64 filter rows so one CTA/thread owns both halves of the gate.
@@ -263,9 +270,14 @@ static int build(dsvc_diffnet* h, const dsvc_diffnet_weights* w, cudaStream_t s)
     DSVC_TRY(upload_f(h->w_dil, wd, s));
     DSVC_TRY(upload_f(h->w_out, wo, s));
   } else {
-    DSVC_TRY(make_f16_pair(h->h_in, w->input_projection_w, (size_t)C * M, s));
+    // mel axis padded to Mp: input projection [C][Mp] with zero columns past M, head [Mp][C] with zero rows past M
+    // (zeros leave the max-abs, so the power-of-two pre-scale, unchanged)
+    std::vector<float> win((size_t)C * Mp, 0.f), whd((size_t)Mp * C, 0.f);
+    for (int c = 0; c < C; ++c) memcpy(&win[(size_t)c * Mp], w->input_projection_w + (size_t)c * M, (size_t)M * 4);
+    memcpy(whd.data(), w->output_projection_w, (size_t)M * C * 4);
+    DSVC_TRY(make_f16_pair(h->h_in, win.data(), win.size(), s));
     DSVC_TRY(make_f16_pair(h->h_skip, w->skip_projection_w, (size_t)C * C, s));
-    DSVC_TRY(make_f16_pair(h->h_head, w->output_projection_w, (size_t)M * C, s));
+    DSVC_TRY(make_f16_pair(h->h_head, whd.data(), whd.size(), s));
     for (int l = 0; l < L; ++l) {
       h->h_dil.emplace_back(new F16Pair());
       h->h_out.emplace_back(new F16Pair());
@@ -304,7 +316,7 @@ static const PlaneBuf& zplane(const dsvc_diffnet* h, int l) { return (h->skip_de
 
 // TMA descriptors of every contraction of the tcgen05 path (depend on B, Tmax and the workspace)
 static int tc_build_maps(dsvc_diffnet* h) {
-  const int M = h->cfg.mel_bins, C = h->cfg.residual_channels, L = h->cfg.residual_layers;
+  const int Mp = h->Mp, C = h->cfg.residual_channels, L = h->cfg.residual_layers;
   const int B = h->B, T = h->Tmax;
   auto gemm = [&](TcGemmMaps& g, const PlaneBuf& a, int K, const F16Pair& w, int rows) -> int {
     DSVC_TRY(tc_make_a_map(&g.a_hi, a.hi.as<__half>(), B, T, K));
@@ -317,9 +329,9 @@ static int tc_build_maps(dsvc_diffnet* h) {
     DSVC_TRY(tc_make_b_map(&g.b64_lo, w.lo.as<__half>(), rows, K, 64));
     return DSVC_OK;
   };
-  DSVC_TRY(gemm(h->maps.in, h->XIN, M, h->h_in, C));
+  DSVC_TRY(gemm(h->maps.in, h->XIN, Mp, h->h_in, C));
   DSVC_TRY(gemm(h->maps.skip, h->SP, C, h->h_skip, C));
-  DSVC_TRY(gemm(h->maps.head, h->R, C, h->h_head, M));
+  DSVC_TRY(gemm(h->maps.head, h->R, C, h->h_head, Mp));
   h->maps.dil.resize(L);
   h->maps.out.resize(L);
   for (int l = 0; l < L; ++l) {
@@ -389,7 +401,7 @@ static EpiSkipProj::Params mk_skip(const dsvc_diffnet* h) {
 static EpiHead::Params mk_head(const dsvc_diffnet* h, const HeadArgs& ha) {
   EpiHead::Params e{};
   e.bias = h->b_head.as<float>(); e.st = h->state.as<StepState>(); e.mode = ha.mode; e.B = h->B; e.Tmax = h->Tmax;
-  e.M = h->cfg.mel_bins; e.out = ha.out; e.xs = h->XS.as<float>(); e.XIN = h->XIN.view(h->tc);
+  e.M = h->cfg.mel_bins; e.Mp = h->Mp; e.out = ha.out; e.xs = h->XS.as<float>(); e.XIN = h->XIN.view(h->tc);
   e.c_recip = h->c_recip.as<float>(); e.c_recipm1 = h->c_recipm1.as<float>(); e.c_coef1 = h->c_coef1.as<float>();
   e.c_coef2 = h->c_coef2.as<float>(); e.c_logvar = h->c_logvar.as<float>();
   e.alphas_cumprod = h->c_acp.as<float>(); e.hist = h->hist.as<float>();
@@ -402,7 +414,7 @@ static EpiHead::Params mk_head(const dsvc_diffnet* h, const HeadArgs& ha) {
 static int enqueue_inproj(dsvc_diffnet* h, int tsel, cudaStream_t s) {
   const int M = h->cfg.mel_bins, C = h->cfg.residual_channels;
   const EpiInProj::Params e = mk_inproj(h, tsel);
-  if (h->tc) return tc_launch<EpiInProj>(h->maps.in, e, h->B, h->Tmax, M, C, 1, 0, h->passes, s, tiles_of(h));
+  if (h->tc) return tc_launch<EpiInProj>(h->maps.in, e, h->B, h->Tmax, h->Mp, C, 1, 0, h->passes, s, tiles_of(h));
   return launch_fp32<EpiInProj>(h, base_params(h->XIN.f32.as<float>(), h->w_in.as<float>(), h->B, h->Tmax, M, C, 1, 0), e, s);
 }
 
@@ -587,32 +599,32 @@ static int enqueue_eval(dsvc_diffnet* h, const HeadArgs& ha, cudaStream_t s) {
   }
   {  // K4b output_projection + sampler update
     const EpiHead::Params e = mk_head(h, ha);
-    if (h->tc) DSVC_TRY(tc_launch<EpiHead>(h->maps.head, e, B, T, C, M, 1, 0, h->passes, s, tiles_of(h)));
+    if (h->tc) DSVC_TRY(tc_launch<EpiHead>(h->maps.head, e, B, T, C, h->Mp, 1, 0, h->passes, s, tiles_of(h)));
     else DSVC_TRY(launch_fp32<EpiHead>(h, base_params(h->R.f32.as<float>(), h->w_head.as<float>(), B, T, C, M, 1, 0), e, s));
   }
   return DSVC_OK;
 }
 
 static int load_x(dsvc_diffnet* h, const float* spec, cudaStream_t s) {
-  // [B][M][T] -> XS [B][T][M] (+ operand plane of input_projection)
-  const int M = h->cfg.mel_bins;
+  // [B][M][T] -> XS [B][T][Mp] (+ operand plane of input_projection); the pad columns M..Mp-1 are not written
+  const int M = h->cfg.mel_bins, Mp = h->Mp;
   dim3 grid(ceil_div(h->Tmax, 32), ceil_div(M, 32), h->B), block(32, 8);
   if (h->packed)
-    pack_rows_kernel<<<grid, block, 0, s>>>(spec, h->XS.as<float>(), h->XIN.view(h->tc), h->rowmap.as<int2>(), h->Tmax, M, h->uT);
+    pack_rows_kernel<<<grid, block, 0, s>>>(spec, h->XS.as<float>(), h->XIN.view(h->tc), h->rowmap.as<int2>(), h->Tmax, M, h->uT, Mp);
   else
-  transpose_kernel<<<grid, block, 0, s>>>(spec, h->XS.as<float>(), h->XIN.view(h->tc), M, h->Tmax);
+  transpose_kernel<<<grid, block, 0, s>>>(spec, h->XS.as<float>(), h->XIN.view(h->tc), M, h->Tmax, h->Tmax, Mp);
   DSVC_LAUNCH_CHECK();
   return DSVC_OK;
 }
 
 static int store_x(dsvc_diffnet* h, float* x, cudaStream_t s) {
-  const int M = h->cfg.mel_bins;
+  const int M = h->cfg.mel_bins, Mp = h->Mp;
   Plane none{nullptr, nullptr, nullptr};
   dim3 grid(ceil_div(M, 32), ceil_div(h->Tmax, 32), h->B), block(32, 8);
   if (h->packed)
-    unpack_rows_kernel<<<dim3(ceil_div(h->Tmax, 32), ceil_div(M, 32)), block, 0, s>>>(h->XS.as<float>(), x, h->rowmap.as<int2>(), h->Tmax, M, h->uT);
+    unpack_rows_kernel<<<dim3(ceil_div(h->Tmax, 32), ceil_div(M, 32)), block, 0, s>>>(h->XS.as<float>(), x, h->rowmap.as<int2>(), h->Tmax, M, h->uT, Mp);
   else
-  transpose_kernel<<<grid, block, 0, s>>>(h->XS.as<float>(), x, none, h->Tmax, M);
+  transpose_kernel<<<grid, block, 0, s>>>(h->XS.as<float>(), x, none, h->Tmax, M, Mp, h->Tmax);
   DSVC_LAUNCH_CHECK();
   return DSVC_OK;
 }
@@ -657,12 +669,12 @@ int dsvc_diffnet_create(dsvc_diffnet_t** out, const dsvc_diffnet_config* cfg, co
   DSVC_REQUIRE(cfg->math == DSVC_MATH_TC3F16 || cfg->math == DSVC_MATH_FP32 || cfg->math == DSVC_MATH_TC1F16,
                "unknown math mode %d", cfg->math);
   if (cfg->math != DSVC_MATH_FP32)
-    DSVC_REQUIRE(M % 64 == 0 && C % 128 == 0, "tensor-core math needs mel_bins %% 64 == 0 and residual_channels %% 128 == 0 "
-                 "(got M=%d C=%d); use DSVC_MATH_FP32", M, C);
+    DSVC_REQUIRE(C % 128 == 0, "tensor-core math needs residual_channels %% 128 == 0 (got C=%d); use DSVC_MATH_FP32", C);
   dsvc_diffnet* h = new dsvc_diffnet();
   h->cfg = *cfg;
   h->tc = cfg->math != DSVC_MATH_FP32;
   h->passes = cfg->math == DSVC_MATH_TC1F16 ? 1 : 3;
+  h->Mp = h->tc ? 64 * ceil_div(M, 64) : M;
   h->pingpong = h->tc && tc_layer_env() > 0;     // fused-layer mode needs the conv-input plane double-buffered
   int r = build(h, w, (cudaStream_t)stream);
   if (r != DSVC_OK) { delete h; return r; }
@@ -732,8 +744,8 @@ int dsvc_diffnet_prepare(dsvc_diffnet_t* h, int32_t B, int32_t Tmax, const int32
   const size_t n = (size_t)B * Tmax;
   DSVC_TRY(h->X.reserve(n * C * 4));
   DSVC_TRY(h->S.reserve(n * C * 4));
-  DSVC_TRY(h->XS.reserve(n * M * 4));
-  DSVC_TRY(h->hist.reserve(4 * n * M * 4));
+  DSVC_TRY(h->XS.reserve(n * h->Mp * 4));
+  DSVC_TRY(h->hist.reserve(4 * n * h->Mp * 4));
   DSVC_TRY(h->CP.reserve((size_t)L * n * 2 * C * 4));
   DSVC_TRY(h->cond_cl.reserve(n * H * 4));
   DSVC_TRY(h->lengths.reserve((size_t)B * 4));
@@ -753,7 +765,13 @@ int dsvc_diffnet_prepare(dsvc_diffnet_t* h, int32_t B, int32_t Tmax, const int32
   DSVC_TRY(h->Z.reserve(n * C, tc));
   DSVC_TRY(h->SP.reserve(n * C, tc));
   DSVC_TRY(h->R.reserve(n * C, tc));
-  DSVC_TRY(h->XIN.reserve(n * M, tc));
+  DSVC_TRY(h->XIN.reserve(n * h->Mp, tc));
+  if (h->Mp != M) {
+    // the input projection's TMA reads all Mp columns of XIN; only the first M are ever written (load_x, head epilogue).
+    // The pad must be zero, not whatever the allocation held: an fp16 NaN times a zero weight is still NaN.
+    DSVC_CUDA(cudaMemsetAsync(h->XIN.hi.p, 0, n * h->Mp * sizeof(__half), s));
+    DSVC_CUDA(cudaMemsetAsync(h->XIN.lo.p, 0, n * h->Mp * sizeof(__half), s));
+  }
   DSVC_CUDA(cudaMemcpyAsync(h->lengths.p, len.data(), (size_t)B * 4, cudaMemcpyHostToDevice, s));
   // Ragged batch on the tensor-core path: only the frame tiles that hold a valid frame do work.  The grid keeps the
   // dense size (a captured graph stays valid whatever the lengths are); dead slots exit at once.  Frames beyond an
@@ -800,9 +818,9 @@ int dsvc_diffnet_prepare(dsvc_diffnet_t* h, int32_t B, int32_t Tmax, const int32
   {
     Plane none{nullptr, nullptr, nullptr};
     dim3 grid(ceil_div(Tmax, 32), ceil_div(H, 32), B), block(32, 8);
-    if (pack) pack_rows_kernel<<<grid, block, 0, s>>>(cond, h->cond_cl.as<float>(), none, h->rowmap.as<int2>(), Tmax, H, user_T);
+    if (pack) pack_rows_kernel<<<grid, block, 0, s>>>(cond, h->cond_cl.as<float>(), none, h->rowmap.as<int2>(), Tmax, H, user_T, H);
     else
-    transpose_kernel<<<grid, block, 0, s>>>(cond, h->cond_cl.as<float>(), none, H, Tmax);
+    transpose_kernel<<<grid, block, 0, s>>>(cond, h->cond_cl.as<float>(), none, H, Tmax, Tmax, H);
     DSVC_LAUNCH_CHECK();
     ConvGemmParams p = base_params(h->cond_cl.as<float>(), h->w_cond.as<float>(), B, Tmax, H, L * 2 * C, 1, 0);
     EpiCondProj::Params e{};

@@ -312,13 +312,15 @@ enum HeadMode : int {
 struct EpiHead {
   static constexpr bool kPair = false;
   struct Params {
-    const float* bias;   // [M]
+    const float* bias;   // [Mp]
     const StepState* st;
     int mode;
-    int B, Tmax, M;
+    int B, Tmax, M;      // M: the model's mel bins -- what the caller's tensors, the noise index and the Philox counter use
+    int Mp;              // row stride of xs / hist / XIN: M padded to whole tiles on the tensor-core path (columns past M:
+                         // zero weights and bias, never stored)
     float wscale;
     float* out;          // HEAD_EVAL: [B,1,M,Tmax]
-    float* xs;           // sampler state x, channels-last [B][Tmax][M]
+    float* xs;           // sampler state x, channels-last [B][Tmax][Mp]
     Plane XIN;           // operand plane of input_projection for the next eval
     const int2* rowmap;  // packed batch: row -> (item, frame) of the caller's layout (noise / Philox / HEAD_EVAL indexing)
     int uB, uT;          // the caller's batch size and Tmax (== B, Tmax when rowmap is null)
@@ -326,7 +328,7 @@ struct EpiHead {
     const float* c_recip; const float* c_recipm1; const float* c_coef1; const float* c_coef2; const float* c_logvar;
     // PLMS
     const float* alphas_cumprod;
-    float* hist;         // [4][B][Tmax][M] eps ring
+    float* hist;         // [4][B][Tmax][Mp] eps ring
   };
 
   // get_x_pred coefficients (diffusion.py:171-177), evaluated in the reference's op order
@@ -354,19 +356,20 @@ struct EpiHead {
     return c;
   }
   __device__ static __forceinline__ void l2_prefetch(const Params& e, int b, int p, int n) {
-    if (e.mode != HEAD_EVAL) l2_prefetch_line(e.xs + ((size_t)b * e.Tmax + p) * e.M + n);
+    if (e.mode != HEAD_EVAL) l2_prefetch_line(e.xs + ((size_t)b * e.Tmax + p) * e.Mp + n);
   }
   __device__ static __forceinline__ EpiPre pre(const Params& e, int b, int p, int n) {
     EpiPre r{};
-    if (e.mode != HEAD_EVAL) r.a = *reinterpret_cast<const float4*>(e.xs + ((size_t)b * e.Tmax + p) * e.M + n);
+    if (e.mode != HEAD_EVAL) r.a = *reinterpret_cast<const float4*>(e.xs + ((size_t)b * e.Tmax + p) * e.Mp + n);
     r.row = e.rowmap ? __ldg(e.rowmap + p) : make_int2(b, p);
     return r;
   }
 
   __device__ static __forceinline__ void apply(const Params& e, int b, int p, int n, const float (&a)[4],
                                                const EpiCol& c, const EpiPre& r) {
+    if (n >= e.M) return;                    // pad columns of the tensor-core path's Mp-wide head tile
     const float eps[4] = {a[0] * e.wscale + c.bias.x, a[1] * e.wscale + c.bias.y, a[2] * e.wscale + c.bias.z, a[3] * e.wscale + c.bias.w};
-    const size_t idx = ((size_t)b * e.Tmax + p) * e.M + n;
+    const size_t idx = ((size_t)b * e.Tmax + p) * e.Mp + n;
     const int ub = r.row.x, up = r.row.y;    // (item, frame) in the caller's [uB][..][uT] tensors
     if (ub < 0) return;                      // padding row of a packed batch: nothing of the caller's lives here
     if (e.mode == HEAD_EVAL) {
@@ -402,7 +405,7 @@ struct EpiHead {
       return;
     }
     // ---- PLMS ----
-    const size_t hs = (size_t)e.B * e.Tmax * e.M;
+    const size_t hs = (size_t)e.B * e.Tmax * e.Mp;
     float dA, cx, ce;
     plms_coefs(e, dA, cx, ce);
     const int head = e.st->head;

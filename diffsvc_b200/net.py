@@ -81,7 +81,7 @@ class DiffNet(nn.Module):
         # --- native state (not part of state_dict) ---
         self.num_timesteps = int(num_timesteps or hparams.get("timesteps", 1000))
         if math_mode is None:
-            tc_ok = in_dims % 64 == 0 and dim % 128 == 0
+            tc_ok = in_dims % 4 == 0 and dim % 128 == 0     # the library pads the mel axis to whole tiles
             math_mode = hparams.get("dsvc_math", "tc3f16" if tc_ok else "fp32")
         self.math_mode = math_mode
         self._h = None

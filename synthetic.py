@@ -22,6 +22,23 @@ NSF_H_44K_V3 = dict(  # a HiFi-GAN "V3"-style 44.1 kHz NSF generator: ResBlock2 
     NSF_H_44K, resblock="2", resblock_kernel_sizes=[3, 5, 7], resblock_dilation_sizes=[[1, 2], [2, 6], [3, 12]])
 
 
+HIFIGAN_H_24K = dict(  # assumed 24 kHz HiFi-GAN topology (SURVEY.md section 8c): its config.yaml is not in the reference repo
+    resblock="1", upsample_rates=[8, 4, 2, 2], upsample_kernel_sizes=[16, 8, 4, 4],
+    upsample_initial_channel=512, resblock_kernel_sizes=[3, 7, 11],
+    resblock_dilation_sizes=[[1, 3, 5], [1, 3, 5], [1, 3, 5]], num_mels=80, sampling_rate=24000,
+    audio_sample_rate=24000, hop_size=128, use_pitch_embed=True)
+
+
+# The 24 kHz model of training/config.yaml (the reference's default config), as overrides of the 44.1 kHz defaults
+# (diffsvc_b200.hparams.DEFAULTS_44K).  spec_min / spec_max stay scalar: the config's per-bin lists are trained statistics.
+HPARAMS_24K = dict(
+    audio_num_mel_bins=80, audio_sample_rate=24000, hop_size=128, fft_size=512, win_size=512, fmin=30, fmax=12000,
+    hidden_size=256, residual_layers=20, residual_channels=256, dilation_cycle_length=4, keep_bins=80,
+    f0_min=50.0, f0_max=1100.0, pndm_speedup=10, use_nsf=True, use_pitch_embed=True,
+    vocoder="diffsvc_b200.vocoders.hifigan.HifiGAN", vocoder_ckpt="checkpoints/0109_hifigan_bigpopcs_hop128",
+)
+
+
 def synth_diffnet_weights(M=128, C=384, H=256, L=20, seed=1234):
     """Seeded synthetic DiffNet state dict with the reference's key names and init statistics
     (kaiming-normal convs net.py:47-50, default Linear init), and a NON-zero output_projection
